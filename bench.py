@@ -9,6 +9,7 @@ A "step" is one forward + one backward of the ring attention op on synthetic q/k
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference     # the unmodified reference from baseline/_ref (Triton + NCCL P2P)
+    python bench.py --dump-outputs DIR   # also write what the last timed step returned, to compare two builds
 
 Timing: CUDA events on the launching stream, barrier + synchronize on both sides, max over ranks.  The
 q/k/v shards (>= 268 MB each) are larger than the 126 MB L2, so no explicit flush is needed.
@@ -31,6 +32,8 @@ import threading
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+
+DUMP_BYTES = 32 * 2 ** 20  # --dump-outputs: float32 bytes over all arrays and ranks
 
 
 def parse_args():
@@ -56,7 +59,32 @@ def parse_args():
     ap.add_argument("--memory", default="auto", choices=["auto", "gather", "ring"],
                     help="ring_cuda.CONFIG['memory']: 'ring' = per-hop launches against a 2-slot K/V window (O(n/W) "
                          "workspace); 'auto' picks it for K/V slots >= 256 MiB per rank (the headline config at any N)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (out, dq, dk, dv of this rank's "
+                         "shard) as float32 DIR/<name>.npy (DIR/<name>_rank<r>.npy for N > 1): the same seeded sample "
+                         f"of token rows on every run, {DUMP_BYTES // 2 ** 20} MiB at most over all ranks")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(out_dir: str, arrays: dict, rank: int, world: int) -> dict:
+    """Write float32 samples of ``arrays`` ([batch, tokens, heads, dim] each): the same token rows of every array, drawn
+    from a fixed seed, as many as fit ``DUMP_BYTES`` over all ranks (all rows when the shard is small enough)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    n = next(iter(arrays.values())).shape[1]
+    row_bytes = sum(t[:, :1].numel() * 4 for t in arrays.values())
+    n_rows = max(1, min(n, DUMP_BYTES // (world * row_bytes)))
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:n_rows].sort().values
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, t in arrays.items():
+        sample = t.detach().index_select(1, rows.to(t.device)).float().cpu().numpy()
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), sample)
+    return {"dir": out_dir, "arrays": sorted(arrays), "token_rows": n_rows, "of": n}
 
 
 class ClockSampler:
@@ -277,7 +305,8 @@ def main():
         fwd = 4.0 * B * H * float(S_) * float(S_) * D * 0.5
         return fwd * (1.0 if args.fwd_only else 3.5)
 
-    def measure(S_: int, steps: int, warmup: int, with_e2e: bool, with_check: bool, sample_clocks: bool):
+    def measure(S_: int, steps: int, warmup: int, with_e2e: bool, with_check: bool, sample_clocks: bool,
+                dump_dir: str | None = None):
         """One configuration: device-timed loop (+ e2e loop, + sampled-row check).  Returns a dict (rank 0 prints)."""
         n_ = S_ // world
         torch.cuda.reset_peak_memory_stats(dev)
@@ -292,14 +321,16 @@ def main():
             return attn(q_, k_, v_, bucket)
 
         def step():
+            """One timed step; returns what a caller receives (the output and, with the backward, dQ / dK / dV)."""
             out = call(q, k, v)
             if args.fwd_only:
-                return out
+                return {"out": out}
             if ref_env:
                 os.environ["DISABLE_MMA_V5"] = "1"  # forward kernels are compiled by now and keep tcgen05
             out.backward(w)
+            res = {"out": out, "dq": q.grad, "dk": k.grad, "dv": v.grad}
             q.grad = k.grad = v.grad = None
-            return out
+            return res
 
         for _ in range(warmup):
             step()
@@ -331,13 +362,16 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         sync()
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):  # no step's results are held while the next one runs
             step()
+        last = step()
         e1.record()
         sync()
         ms = max_over_ranks(e0.elapsed_time(e1))
         clocks = sampler.stop() if (rank == 0 and sample_clocks) else None
         n_launch = launches["count"] - launches_before
+        dumped = dump_outputs(dump_dir, last, rank, world) if dump_dir else None
+        del last
 
         flops_per_step = flops_of(S_)
         row = {
@@ -352,6 +386,8 @@ def main():
             "clocks": clocks,
         }
         row["hop_window"] = bool(hop_window)
+        if dumped:
+            row["dumped_outputs"] = dumped
         if args.impl == "ours":
             # device memory: caching-allocator peak + the symmetric (cudaMalloc / IPC) workspace of the ring
             symm = 0
@@ -507,7 +543,8 @@ def main():
 
     try:
         main_row = measure(S, args.steps, args.warmup, with_e2e=not args.no_e2e,
-                           with_check=(args.check != "off" and args.impl == "ours"), sample_clocks=True)
+                           with_check=(args.check != "off" and args.impl == "ours"), sample_clocks=True,
+                           dump_dir=args.dump_outputs)
     except BaseException as e:  # noqa: BLE001
         if args.impl == "reference":
             unavailable(f"reference failed to run: {type(e).__name__}: {e}")
@@ -568,6 +605,7 @@ def main():
             **({"ring_kv_gbps": main_row["ring_kv_gbps"]} if "ring_kv_gbps" in main_row else {}),
             **({"check": main_row["check"]} if "check" in main_row else {}),
             **({"memory_gb": main_row["memory_gb"]} if "memory_gb" in main_row else {}),
+            **({"dumped_outputs": main_row["dumped_outputs"]} if "dumped_outputs" in main_row else {}),
             "rows": rows,
         }
         print(json.dumps(line))

@@ -1,97 +1,84 @@
-"""Side-by-side parity with the UNMODIFIED reference package (installed once into ``baseline/_ref``, see DESIGN.md §6).
+"""Side-by-side parity with the original ring-attention-pytorch (0.5.20) on its CPU code path.
 
-The reference's CPU code path needs neither Triton nor a GPU, so the modules can be compared directly: a reference
-``state_dict`` must load into the rebuilt modules unchanged and produce the same numbers.  Skipped when the reference
-install is not present (it is git-ignored).
+A ``state_dict`` of the original's modules must load into the rebuilt modules unchanged and produce the same numbers,
+and every public callable of the original must exist here with compatible parameters.  What the original computed is
+stored in ``tests/golden/``: ``reference_parity.npz`` holds the inputs, the original's weights and its outputs and
+gradients, ``reference_api.json`` the parameter lists of its public callables.  So these tests need nothing outside
+the repository.  To regenerate both files from a checkout of the original (it needs einops, beartype and jaxtyping):
+
+    python tests/test_reference_parity.py --write-golden /path/to/ring-attention-pytorch
 """
+import json
 import os
 import sys
+import tempfile
 
+import numpy as np
 import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
+GOLDEN_NPZ = os.path.join(ROOT, "tests", "golden", "reference_parity.npz")
+GOLDEN_API = os.path.join(ROOT, "tests", "golden", "reference_api.json")
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "ring_attention_pytorch")),
-                                reason="reference package not installed in baseline/_ref")
+TRANSFORMER_KW = dict(num_tokens=64, dim=32, depth=2, causal=True, dim_head=8, heads=4, num_grouped_query_heads=2,
+                      bucket_size=4, ring_attn=False, use_cuda_kernel=False)
+ATTENTION_KW = dict(dim=32, dim_head=8, heads=4, num_grouped_query_heads=2, bucket_size=4, ring_attn=False,
+                    rotary_embed=True, use_cuda_kernel=False)
+RING_TRANSFORMER_KW = dict(num_tokens=64, dim=32, depth=2, causal=True, dim_head=8, heads=4, num_grouped_query_heads=2,
+                           bucket_size=4, ring_attn=True, ring_seq_size=8, use_cuda_kernel=False)
+# (module of the original, module here, public names compared)
+API_MODULES = {
+    "": "ring_attention_pytorch_b200",
+    "distributed": "ring_attention_pytorch_b200.parallel.distributed",
+    "ring": "ring_attention_pytorch_b200.parallel.ring",
+    "zig_zag_attention": "ring_attention_pytorch_b200.ops.zig_zag",
+}
+API_NAMES = {
+    "": ["RingAttention", "RingTransformer", "RingRotaryEmbedding", "apply_rotary_pos_emb", "default_attention",
+         "ring_flash_attn", "ring_flash_attn_cuda", "tree_attn_decode"],
+    "distributed": ["all_gather_variable_dim", "split_by_rank", "get_rank", "get_world_size", "is_distributed",
+                    "pad_dim_to"],
+    "ring": ["ring_pass", "all_ring_pass", "null_ring_pass", "one_ring_pass", "get_rank", "get_world_size"],
+    "zig_zag_attention": ["zig_zag_pad_seq", "zig_zag_shard", "zig_zag_attn"],
+}
+
+
+def load_golden() -> dict:
+    """Golden arrays by name; float16 entries are float32 values that half precision holds exactly."""
+    with np.load(GOLDEN_NPZ) as z:
+        return {k: torch.from_numpy(z[k].astype(np.float32) if z[k].dtype == np.float16 else z[k]) for k in z.files}
+
+
+def _sub(golden: dict, prefix: str) -> dict:
+    return {k[len(prefix):]: v for k, v in golden.items() if k.startswith(prefix)}
+
+
+def _params(fn):
+    import inspect
+
+    target = fn.__init__ if inspect.isclass(fn) else fn
+    try:
+        sig = inspect.signature(target)
+    except (TypeError, ValueError):
+        return None
+    return [p for p in sig.parameters if p not in ("self", "args", "kwargs")]
 
 
 @pytest.fixture(scope="module")
 def ref():
-    sys.path.insert(0, REF)
-    try:
-        import ring_attention_pytorch as pkg
-        import ring_attention_pytorch.ring_attention  # noqa: F401
-        import ring_attention_pytorch.tree_attn_decoding  # noqa: F401
-    except Exception as e:  # pragma: no cover - depends on the image
-        pytest.skip(f"reference package does not import here: {e}")
-    finally:
-        sys.path.remove(REF)
-    return pkg
+    return load_golden()
 
 
-def test_transformer_loads_reference_checkpoint_and_matches(ref):
-    from ring_attention_pytorch_b200 import RingTransformer
+def _run_distributed(*args, **kwargs):
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from dist_utils import run_distributed
 
-    torch.manual_seed(0)
-    kw = dict(num_tokens=64, dim=32, depth=2, causal=True, dim_head=8, heads=4, num_grouped_query_heads=2,
-              bucket_size=4, ring_attn=False, use_cuda_kernel=False)
-    theirs = ref.RingTransformer(**kw)
-    ours = RingTransformer(**kw)
-    ours.load_state_dict(theirs.state_dict())  # strict: identical parameter names and shapes
-    x = torch.randint(0, 64, (2, 17))
-    assert torch.allclose(ours(x), theirs(x), atol=1e-5)
-    la, lb = ours(x, return_loss=True), theirs(x, return_loss=True)
-    assert torch.allclose(la, lb, atol=1e-6)
-    la.backward()
-    lb.backward()
-    for (n, a), (_, b) in zip(ours.named_parameters(), theirs.named_parameters()):
-        assert torch.allclose(a.grad, b.grad, atol=1e-5), n
+    run_distributed(*args, **kwargs)
 
 
-@pytest.mark.parametrize("causal", [False, True])
-def test_attention_module_matches(ref, causal):
-    from ring_attention_pytorch_b200 import RingAttention
-
-    torch.manual_seed(1)
-    kw = dict(dim=32, dim_head=8, heads=4, num_grouped_query_heads=2, causal=causal, bucket_size=4, ring_attn=False,
-              rotary_embed=True, use_cuda_kernel=False)
-    theirs, ours = ref.RingAttention(**kw), RingAttention(**kw)
-    ours.load_state_dict(theirs.state_dict())
-    x = torch.randn(2, 19, 32)
-    mask = None if causal else (torch.rand(2, 19) > 0.25)
-    assert torch.allclose(ours(x, mask), theirs(x, mask), atol=1e-5)
-
-
-def test_functional_ops_match(ref):
-    from ring_attention_pytorch_b200 import (RingRotaryEmbedding, apply_rotary_pos_emb, default_attention,
-                                             ring_flash_attn, tree_attn_decode)
-
-    torch.manual_seed(2)
-    q = torch.randn(2, 21, 4, 8, requires_grad=True)
-    k = torch.randn(2, 21, 2, 8, requires_grad=True)
-    v = torch.randn(2, 21, 2, 8, requires_grad=True)
-    mask = torch.rand(2, 21) > 0.3
-    for causal in (False, True):
-        m = None if causal else mask
-        a = default_attention(q, k, v, m, causal)
-        b = ref.default_attention(q, k, v, m, causal)
-        assert torch.allclose(a, b, atol=1e-5)
-        # naive flash op, single process: forward and all three gradients (the reference's dK/dV defect needs a ring)
-        fa = ring_flash_attn(q, k, v, m, causal, 4)
-        fb = ref.ring_flash_attn(q, k, v, m, causal, 4)
-        assert torch.allclose(fa, fb, atol=1e-5)
-        g = torch.randn_like(fa)
-        for x, y in zip(torch.autograd.grad(fa, (q, k, v), g), torch.autograd.grad(fb, (q, k, v), g)):
-            assert torch.allclose(x, y, atol=1e-4)
-
-    rot_a, rot_b = RingRotaryEmbedding(8), ref.RingRotaryEmbedding(8)
-    pa, pb = rot_a(21), rot_b(21)
-    assert torch.allclose(pa, pb, atol=1e-6)
-    assert torch.allclose(apply_rotary_pos_emb(pa, q), ref.ring_attention.apply_rotary_pos_emb(pb, q), atol=1e-6)
-
-    # the reference's decode needs an initialised process group even for one rank (ours does not)
+def _one_rank_group():
+    """A single-process gloo group (the original's decode needs one even for one rank; ours runs inside it too)."""
     import socket
 
     import torch.distributed as dist
@@ -100,145 +87,317 @@ def test_functional_ops_match(ref):
         sock.bind(("127.0.0.1", 0))
         port = sock.getsockname()[1]
     dist.init_process_group("gloo", init_method=f"tcp://127.0.0.1:{port}", rank=0, world_size=1)
+
+
+def test_transformer_loads_reference_checkpoint_and_matches(ref):
+    from ring_attention_pytorch_b200 import RingTransformer
+
+    g = _sub(ref, "transformer/")
+    ours = RingTransformer(**TRANSFORMER_KW)
+    ours.load_state_dict(_sub(g, "state/"))  # strict: identical parameter names and shapes
+    x = g["x"]
+    assert torch.allclose(ours(x), g["logits"], atol=1e-5)
+    la = ours(x, return_loss=True)
+    assert torch.allclose(la, g["loss"], atol=1e-6)
+    la.backward()
+    grads = _sub(g, "grad/")
+    assert sorted(grads) == sorted(n for n, _ in ours.named_parameters())
+    for n, a in ours.named_parameters():
+        assert torch.allclose(a.grad, grads[n], atol=1e-5), n
+
+
+@pytest.mark.parametrize("causal", [False, True])
+def test_attention_module_matches(ref, causal):
+    from ring_attention_pytorch_b200 import RingAttention
+
+    g = _sub(ref, f"attention_causal{int(causal)}/")
+    ours = RingAttention(causal=causal, **ATTENTION_KW)
+    ours.load_state_dict(_sub(ref, "attention/state/"))  # one set of weights for both settings
+    mask = g.get("mask")
+    assert (mask is None) == causal
+    assert torch.allclose(ours(g["x"], mask), g["out"], atol=1e-5)
+
+
+def test_functional_ops_match(ref):
+    from ring_attention_pytorch_b200 import (RingRotaryEmbedding, apply_rotary_pos_emb, default_attention,
+                                             ring_flash_attn, tree_attn_decode)
+
+    g = _sub(ref, "functional/")
+    q, k, v = (g[n].clone().requires_grad_() for n in "qkv")
+    for causal in (False, True):
+        m = None if causal else g["mask"]
+        a = default_attention(q, k, v, m, causal)
+        assert torch.allclose(a, g[f"causal{int(causal)}/default"], atol=1e-5)
+        # naive flash op, single process: forward and all three gradients (the original's dK/dV defect needs a ring)
+        fa = ring_flash_attn(q, k, v, m, causal, 4)
+        assert torch.allclose(fa, g[f"causal{int(causal)}/flash"], atol=1e-5)
+        grads = torch.autograd.grad(fa, (q, k, v), g[f"causal{int(causal)}/dout"])
+        for name, x in zip("qkv", grads):
+            assert torch.allclose(x, g[f"causal{int(causal)}/d{name}"], atol=1e-4)
+
+    pa = RingRotaryEmbedding(8)(21)
+    assert torch.allclose(pa, g["rotary/pos"], atol=1e-6)
+    assert torch.allclose(apply_rotary_pos_emb(pa, q), g["rotary/q"], atol=1e-6)
+
+    import torch.distributed as dist
+
+    _one_rank_group()
     try:
-        dq, dk, dv = torch.randn(2, 4, 1, 8), torch.randn(2, 4, 33, 8), torch.randn(2, 4, 33, 8)
-        want = ref.tree_attn_decode(dq, dk, dv, use_triton=False)
-        assert torch.allclose(tree_attn_decode(dq, dk, dv), want, atol=1e-5)
+        assert torch.allclose(tree_attn_decode(g["decode/q"], g["decode/k"], g["decode/v"]), g["decode/out"], atol=1e-5)
     finally:
         dist.destroy_process_group()
 
 
 def _zigzag_parity_worker(rank, world):
-    """zig-zag helpers against the reference's, inside a real gloo group (the reference shards by global rank)."""
-    sys.path.insert(0, REF)
-    from ring_attention_pytorch import zig_zag_attention as theirs
-
+    """zig-zag helpers against the original's, inside a real gloo group (the original shards by global rank)."""
     from ring_attention_pytorch_b200.ops import zig_zag as ours
 
-    torch.manual_seed(0)
-    x = torch.randn(2, 29, 16)
+    g = _sub(load_golden(), "zigzag/")
+    r = _sub(g, f"rank{rank}/")
+    x = g["x"]
     pa, inv_a = ours.zig_zag_pad_seq(x)
-    pb, inv_b = theirs.zig_zag_pad_seq(x)
-    assert torch.equal(pa, pb)
+    assert torch.equal(pa, g["padded"])
     (sa, qa, ka), gather_a = ours.zig_zag_shard(pa)
-    (sb, qb, kb), gather_b = theirs.zig_zag_shard(pb)
-    assert torch.equal(sa, sb) and torch.equal(qa, qb) and torch.equal(ka, kb)
-    assert torch.equal(inv_a(gather_a(sa)), inv_b(gather_b(sb))) and torch.equal(inv_a(gather_a(sa)), x)
+    assert torch.equal(sa, r["shard"]) and torch.equal(qa, r["q_pos"]) and torch.equal(ka, r["k_pos"])
+    assert torch.equal(inv_a(gather_a(sa)), x)
 
-    # attention on the shard with the caller-built dense mask (the reference's only mode) and with our ring schedule
-    h, d = 4, 8
-    q = torch.randn(2, h, sa.shape[1], d)
-    k = torch.randn(2, 2, sa.shape[1], d)
-    v = torch.randn(2, 2, sa.shape[1], d)
+    # attention on the shard with the caller-built dense mask (the original's only mode) and with our ring schedule
+    q, k, v = g["q"], g["k"], g["v"]
     mask = qa[:, None] >= ka[None, :]
-    want = theirs.zig_zag_attn(q, k, v, attn_mask=mask)
-    assert torch.allclose(ours.zig_zag_attn(q, k, v, attn_mask=mask), want, atol=1e-5)
-    assert torch.allclose(ours.zig_zag_attn(q, k, v, causal=True), want, atol=1e-5)
+    assert torch.allclose(ours.zig_zag_attn(q, k, v, attn_mask=mask), r["out"], atol=1e-5)
+    assert torch.allclose(ours.zig_zag_attn(q, k, v, causal=True), r["out"], atol=1e-5)
 
 
 def test_zig_zag_matches_reference(ref):
-    sys.path.insert(0, os.path.join(ROOT, "tests"))
-    from dist_utils import run_distributed
-
-    run_distributed(_zigzag_parity_worker, 2)
+    _run_distributed(_zigzag_parity_worker, 2)
 
 
 def _ring_transformer_parity_worker(rank, world, striped):
-    """Sequence-parallel forward of the two RingTransformers with the same weights (forward only: the reference's ring
+    """Sequence-parallel forward of the original's weights in our RingTransformer (forward only: the original's ring
     backward returns wrong dK/dV, SURVEY D1).  The two packages stripe differently on the CPU path, but both undo their
     permutation on the way out, so the logits must agree."""
-    sys.path.insert(0, REF)
-    import ring_attention_pytorch as theirs
-
     from ring_attention_pytorch_b200 import RingTransformer
 
-    torch.manual_seed(0)
-    kw = dict(num_tokens=64, dim=32, depth=2, causal=True, dim_head=8, heads=4, num_grouped_query_heads=2, bucket_size=4,
-              ring_attn=True, striped_ring_attn=striped, ring_seq_size=8, use_cuda_kernel=False)
-    a, b = RingTransformer(**kw), theirs.RingTransformer(**kw)
-    a.load_state_dict(b.state_dict())
-    torch.manual_seed(1)
-    x = torch.randint(0, 64, (2, 15))  # padded to 16 = 2 ranks x ring_seq_size 8
+    golden = load_golden()
+    g = _sub(golden, f"ring_transformer_striped{int(striped)}/")
+    a = RingTransformer(striped_ring_attn=striped, **RING_TRANSFORMER_KW)
+    a.load_state_dict(_sub(golden, "transformer/state/"))  # the single-process transformer's weights
     with torch.no_grad():
-        la, lb = a(x), b(x)
+        la = a(g["x"])  # padded to 16 = 2 ranks x ring_seq_size 8
+    lb = g["logits"]  # every rank of the original returned the same logits
     assert la.shape == lb.shape
     assert torch.allclose(la, lb, atol=1e-4), (la - lb).abs().max()
 
 
 @pytest.mark.parametrize("striped", [False, True])
 def test_ring_transformer_forward_matches_reference_under_gloo(ref, striped):
-    sys.path.insert(0, os.path.join(ROOT, "tests"))
-    from dist_utils import run_distributed
-
-    run_distributed(_ring_transformer_parity_worker, 2, striped)
+    _run_distributed(_ring_transformer_parity_worker, 2, striped)
 
 
 def _tree_parity_worker(rank, world, seq_len):
-    sys.path.insert(0, REF)
-    import ring_attention_pytorch as theirs
-
     from ring_attention_pytorch_b200 import tree_attn_decode
 
-    torch.manual_seed(0)  # identical inputs on every rank; both implementations shard K/V by rank internally
-    q, k, v = torch.randn(2, 4, 1, 8), torch.randn(2, 4, seq_len, 8), torch.randn(2, 4, seq_len, 8)
-    want = theirs.tree_attn_decode(q, k, v, use_triton=False)
-    assert torch.allclose(tree_attn_decode(q, k, v), want, atol=1e-5)
+    g = _sub(load_golden(), f"tree_decode_n{seq_len}/")  # identical inputs on every rank; K/V are sharded by rank
+    assert torch.allclose(tree_attn_decode(g["q"], g["k"], g["v"]), g["out"], atol=1e-5)
 
 
 @pytest.mark.parametrize("seq_len", [2, 31])  # 2 < world: some ranks hold no keys at all
 def test_tree_decode_matches_reference_under_gloo(ref, seq_len):
-    sys.path.insert(0, os.path.join(ROOT, "tests"))
-    from dist_utils import run_distributed
-
-    run_distributed(_tree_parity_worker, 3, seq_len)
+    _run_distributed(_tree_parity_worker, 3, seq_len)
 
 
-def test_public_api_surface_is_a_superset_of_the_reference(ref):
-    """Every public callable the reference exports exists here under the same name and accepts (at least) the same
-    parameters in the same order, so that call sites written against the reference keep working."""
-    import inspect
+def test_public_api_surface_is_a_superset_of_the_reference():
+    """Every public callable the original exports exists here under the same name and accepts (at least) the same
+    parameters in the same order, so that call sites written against the original keep working."""
+    import importlib
 
     import ring_attention_pytorch_b200 as ours
 
-    ref_mods = {"": ref}
-    sys.path.insert(0, REF)
-    try:
-        import ring_attention_pytorch.distributed as r_dist
-        import ring_attention_pytorch.ring as r_ring
-        import ring_attention_pytorch.zig_zag_attention as r_zz
-    finally:
-        sys.path.remove(REF)
-    import ring_attention_pytorch_b200.ops.zig_zag as o_zz
-    import ring_attention_pytorch_b200.parallel.distributed as o_dist
-    import ring_attention_pytorch_b200.parallel.ring as o_ring
-
-    def params(fn):
-        target = fn.__init__ if inspect.isclass(fn) else fn
-        try:
-            sig = inspect.signature(target)
-        except (TypeError, ValueError):
-            return None
-        return [p for p in sig.parameters if p not in ("self", "args", "kwargs")]
-
+    with open(GOLDEN_API) as f:
+        theirs = json.load(f)
+    assert sorted(theirs) == sorted(API_MODULES)
     checked = 0
-    pairs = [(ref, ours, ["RingAttention", "RingTransformer", "RingRotaryEmbedding", "apply_rotary_pos_emb",
-                          "default_attention", "ring_flash_attn", "ring_flash_attn_cuda", "tree_attn_decode"]),
-             (r_dist, o_dist, ["all_gather_variable_dim", "split_by_rank", "get_rank", "get_world_size",
-                               "is_distributed", "pad_dim_to"]),
-             (r_ring, o_ring, ["ring_pass", "all_ring_pass", "null_ring_pass", "one_ring_pass", "get_rank",
-                               "get_world_size"]),
-             (r_zz, o_zz, ["zig_zag_pad_seq", "zig_zag_shard", "zig_zag_attn"])]
-    for rmod, omod, names in pairs:
-        for name in names:
-            if not hasattr(rmod, name):
-                continue  # the installed reference version does not have it
+    for key, names in theirs.items():
+        omod = importlib.import_module(API_MODULES[key])
+        for name, rp in names.items():
             assert hasattr(omod, name), f"{omod.__name__} lacks {name}"
-            rp, op = params(getattr(rmod, name)), params(getattr(omod, name))
+            op = _params(getattr(omod, name))
             if rp is None or op is None:
                 continue
             assert op[:len(rp)] == rp or set(rp) <= set(op), (name, rp, op)
             checked += 1
     assert checked >= 12
-    # autograd-function entry points are exported under the reference's names as well
+    # autograd-function entry points are exported under the original's names as well
     for name in ("ring_flash_attn_", "ring_flash_attn_cuda_"):
         assert hasattr(ours, name) or name == "ring_flash_attn_cuda_"
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# regeneration of the golden data from the original
+# ------------------------------------------------------------------------------------------------------------------
+def _half(t):
+    """Rounded to values that float16 holds exactly, so that the golden file stores them in half the space."""
+    return t.detach().half().float()
+
+
+def _half_params(module):
+    with torch.no_grad():
+        for p in module.parameters():
+            p.copy_(_half(p))
+    return module
+
+
+def _state(prefix: str, module) -> dict:
+    return {prefix + n: t for n, t in module.state_dict().items()}
+
+
+def _golden_zigzag_worker(rank, world, out_dir):
+    from ring_attention_pytorch import zig_zag_attention as theirs
+
+    torch.manual_seed(0)
+    x = _half(torch.randn(2, 29, 16))
+    pb, _ = theirs.zig_zag_pad_seq(x)
+    (sb, qb, kb), _ = theirs.zig_zag_shard(pb)
+    q = _half(torch.randn(2, 4, sb.shape[1], 8))
+    k = _half(torch.randn(2, 2, sb.shape[1], 8))
+    v = _half(torch.randn(2, 2, sb.shape[1], 8))
+    out = theirs.zig_zag_attn(q, k, v, attn_mask=qb[:, None] >= kb[None, :])
+    res = {"x": x, "padded": pb, "q": q, "k": k, "v": v}
+    res.update({f"rank{rank}/{n}": t for n, t in dict(shard=sb, q_pos=qb, k_pos=kb, out=out).items()})
+    torch.save(res, os.path.join(out_dir, f"rank{rank}.pt"))
+
+
+def _golden_ring_transformer_worker(rank, world, striped, state, out_dir):
+    import ring_attention_pytorch as theirs
+
+    b = theirs.RingTransformer(striped_ring_attn=striped, **RING_TRANSFORMER_KW)
+    b.load_state_dict(state)
+    torch.manual_seed(1)
+    x = torch.randint(0, 64, (2, 15))
+    with torch.no_grad():
+        logits = b(x)
+    torch.save({"x": x, "logits": logits}, os.path.join(out_dir, f"rank{rank}.pt"))
+
+
+def _golden_tree_worker(rank, world, seq_len, out_dir):
+    import ring_attention_pytorch as theirs
+
+    torch.manual_seed(0)
+    q, k, v = (_half(torch.randn(2, 4, n, 8)) for n in (1, seq_len, seq_len))
+    out = theirs.tree_attn_decode(q, k, v, use_triton=False)
+    torch.save({"q": q, "k": k, "v": v, "out": out}, os.path.join(out_dir, f"rank{rank}.pt"))
+
+
+def _golden_distributed(out: dict, prefix: str, worker, world: int, *args) -> None:
+    """Run ``worker`` of the original on ``world`` gloo ranks and merge what every rank saved under ``prefix``; a name
+    that several ranks save is stored once and must be the same on all of them."""
+    with tempfile.TemporaryDirectory() as tmp:
+        _run_distributed(worker, world, *args, tmp)
+        for r in range(world):
+            for n, t in torch.load(os.path.join(tmp, f"rank{r}.pt")).items():
+                if prefix + n in out:
+                    assert torch.equal(out[prefix + n], t), f"ranks of the original disagree on {prefix + n}"
+                out[prefix + n] = t
+
+
+def _compact(t):
+    a = t.detach().numpy()
+    if a.dtype == np.float32 and np.array_equal(a.astype(np.float16).astype(np.float32), a):
+        return a.astype(np.float16)
+    return a
+
+
+def write_golden(reference_root: str) -> None:
+    sys.path.insert(0, reference_root)
+    import ring_attention_pytorch as ref
+    import ring_attention_pytorch.distributed  # noqa: F401
+    import ring_attention_pytorch.ring  # noqa: F401
+    import ring_attention_pytorch.zig_zag_attention  # noqa: F401
+
+    out = {}
+
+    torch.manual_seed(0)
+    transformer = _half_params(ref.RingTransformer(**TRANSFORMER_KW))
+    x = torch.randint(0, 64, (2, 17))
+    out.update(_state("transformer/state/", transformer))
+    out["transformer/x"] = x
+    out["transformer/logits"] = transformer(x)
+    loss = transformer(x, return_loss=True)
+    loss.backward()
+    out["transformer/loss"] = loss
+    for n, p in transformer.named_parameters():
+        out["transformer/grad/" + n] = p.grad
+
+    torch.manual_seed(1)
+    attention = _half_params(ref.RingAttention(causal=False, **ATTENTION_KW))
+    out.update(_state("attention/state/", attention))
+    for causal in (False, True):
+        p = f"attention_causal{int(causal)}/"
+        theirs = ref.RingAttention(causal=causal, **ATTENTION_KW)
+        theirs.load_state_dict(attention.state_dict())
+        x = _half(torch.randn(2, 19, 32))
+        mask = None if causal else (torch.rand(2, 19) > 0.25)
+        out[p + "x"] = x
+        if mask is not None:
+            out[p + "mask"] = mask
+        out[p + "out"] = theirs(x, mask)
+
+    p = "functional/"
+    torch.manual_seed(2)
+    q = _half(torch.randn(2, 21, 4, 8)).requires_grad_()
+    k = _half(torch.randn(2, 21, 2, 8)).requires_grad_()
+    v = _half(torch.randn(2, 21, 2, 8)).requires_grad_()
+    mask = torch.rand(2, 21) > 0.3
+    out.update({p + "q": q, p + "k": k, p + "v": v, p + "mask": mask})
+    for causal in (False, True):
+        c = f"{p}causal{int(causal)}/"
+        m = None if causal else mask
+        out[c + "default"] = ref.default_attention(q, k, v, m, causal)
+        fb = ref.ring_flash_attn(q, k, v, m, causal, 4)
+        dout = _half(torch.randn_like(fb))
+        out[c + "flash"], out[c + "dout"] = fb, dout
+        for name, t in zip("qkv", torch.autograd.grad(fb, (q, k, v), dout)):
+            out[c + "d" + name] = t
+    pb = ref.RingRotaryEmbedding(8)(21)
+    out[p + "rotary/pos"] = pb
+    out[p + "rotary/q"] = ref.ring_attention.apply_rotary_pos_emb(pb, q)
+    import torch.distributed as dist
+
+    _one_rank_group()
+    try:
+        dq, dk, dv = (_half(torch.randn(2, 4, n, 8)) for n in (1, 33, 33))
+        out.update({p + "decode/q": dq, p + "decode/k": dk, p + "decode/v": dv,
+                    p + "decode/out": ref.tree_attn_decode(dq, dk, dv, use_triton=False)})
+    finally:
+        dist.destroy_process_group()
+
+    _golden_distributed(out, "zigzag/", _golden_zigzag_worker, 2)
+    for striped in (False, True):
+        _golden_distributed(out, f"ring_transformer_striped{int(striped)}/", _golden_ring_transformer_worker, 2,
+                            striped, transformer.state_dict())
+    for seq_len in (2, 31):
+        _golden_distributed(out, f"tree_decode_n{seq_len}/", _golden_tree_worker, 3, seq_len)
+
+    os.makedirs(os.path.dirname(GOLDEN_NPZ), exist_ok=True)
+    np.savez_compressed(GOLDEN_NPZ, **{n: _compact(t) for n, t in sorted(out.items())})
+
+    api = {}
+    for key, names in API_NAMES.items():
+        rmod = sys.modules["ring_attention_pytorch" + (f".{key}" if key else "")]
+        # a name the original does not export is left out
+        api[key] = {name: _params(getattr(rmod, name)) for name in names if hasattr(rmod, name)}
+    with open(GOLDEN_API, "w") as f:
+        json.dump(api, f, indent=1)
+        f.write("\n")
+
+
+if __name__ == "__main__":
+    import argparse
+
+    ap = argparse.ArgumentParser(description="regenerate tests/golden/reference_parity.npz and reference_api.json")
+    ap.add_argument("--write-golden", metavar="REFERENCE_ROOT", required=True,
+                    help="checkout of the original ring-attention-pytorch (the directory that holds "
+                         "ring_attention_pytorch/)")
+    args = ap.parse_args()
+    sys.path.insert(0, ROOT)
+    write_golden(os.path.abspath(args.write_golden))
