@@ -378,8 +378,12 @@ __device__ __forceinline__ uint32_t scale_packed(uint32_t w, float f) {
   }
 }
 
-// POLYQ of every 4 logit pairs take their exponential on the FMA pipe (poly_exp2x2) instead of the MUFU.
-template <int D, bool BF16, int POLYQ>
+// POLYQ of every 4 logit pairs take their exponential on the FMA pipe (poly_exp2x2) instead of the MUFU.  Measured on
+// a B200 at n=65536, h=8, causal with none / a quarter / half of them there: 926 / 976 / 957 TFLOP/s (the MUFU phase of
+// a softmax warp shrinks; at one half the extra FMA-pipe instructions start to cost more than the MUFU time they save).
+constexpr int POLYQ = 1;
+
+template <int D, bool BF16>
 __device__ __forceinline__ void softmax_role(FwdSmem<D>& sm, const AttnFwdParams& p, const int t, uint32_t tmem) {
   const int wg_tid = threadIdx.x - 128 * t;
   const uint32_t lane_off = uint32_t((wg_tid / 32) * 32) << 16;
@@ -633,7 +637,7 @@ __device__ __forceinline__ void softmax_role(FwdSmem<D>& sm, const AttnFwdParams
   }
 }
 
-template <int D, bool BF16, int POLYQ>
+template <int D, bool BF16>
 __global__ void __launch_bounds__(NTHREADS, 1)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_kv,
                 const __grid_constant__ AttnFwdParams p) {
@@ -686,7 +690,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
     }
   } else {
     setmaxnreg_inc<192>();
-    softmax_role<D, BF16, POLYQ>(sm, p, warp < 4 ? 0 : 1, tmem);
+    softmax_role<D, BF16>(sm, p, warp < 4 ? 0 : 1, tmem);
   }
 
   tc_fence_before();
@@ -703,18 +707,8 @@ size_t attn_fwd_smem_bytes(int head_dim) {
 template <int D>
 void launch_attn_fwd(const CUtensorMap& map_q, const CUtensorMap& map_kv, const AttnFwdParams& p, int num_sms,
                      cudaStream_t stream) {
-  // RAB_FWD_EXP_POLY = 0 | 1 (default) | 2: none / a quarter / half of the softmax exponentials on the FMA pipe.
-  // Measured at n=65536, h=8, causal: 926 / 976 / 957 TFLOP/s (the MUFU phase of a softmax warp shrinks; at one half
-  // the extra FMA-pipe instructions start to cost more than the MUFU time they save).
-  static const int polyq = [] {
-    const char* e = std::getenv("RAB_FWD_EXP_POLY");
-    return (e != nullptr && e[0] >= '0' && e[0] <= '2') ? int(e[0] - '0') : 1;
-  }();
   using Kern = void (*)(const CUtensorMap, const CUtensorMap, const AttnFwdParams);
-  Kern kern;
-  if (polyq == 2) kern = p.is_bf16 ? attn_fwd_kernel<D, true, 2> : attn_fwd_kernel<D, false, 2>;
-  else if (polyq == 1) kern = p.is_bf16 ? attn_fwd_kernel<D, true, 1> : attn_fwd_kernel<D, false, 1>;
-  else kern = p.is_bf16 ? attn_fwd_kernel<D, true, 0> : attn_fwd_kernel<D, false, 0>;
+  const Kern kern = p.is_bf16 ? attn_fwd_kernel<D, true> : attn_fwd_kernel<D, false>;
   const size_t smem = sizeof(FwdSmem<D>) + 1024;
   cuda_check(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
              "attn_fwd smem attribute");

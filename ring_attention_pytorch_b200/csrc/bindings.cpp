@@ -97,20 +97,6 @@ Tensor umma_probe(const Tensor& a, const Tensor& b, int64_t mode, int64_t n, int
   return out;
 }
 
-// ---------------------------------------------------------------------------------------------
-// fused ring attention forward
-// ---------------------------------------------------------------------------------------------
-void fill_posmap(rab::PosMap& pm, int64_t stride, int64_t seg_len, at::IntArrayRef base0, at::IntArrayRef base1,
-                 int world) {
-  pm.stride = (int)stride;
-  pm.seg_len = (int)seg_len;
-  TORCH_CHECK((int)base0.size() == world && (int)base1.size() == world, "position map needs one base per rank");
-  for (int i = 0; i < rab::kMaxWorld; ++i) {
-    pm.base0[i] = i < world ? (int)base0[i] : 0;
-    pm.base1[i] = i < world ? (int)base1[i] : 0;
-  }
-}
-
 // cycles for `reps` back-to-back tcgen05.mma of one flavour on `ctas` SMs: returns [ctas, 2] (total, issue-side)
 Tensor umma_rate(int64_t mode, int64_t n, int64_t reps, int64_t alt, int64_t ctas) {
   TORCH_CHECK(n == 64 || n == 128 || n == 256, "n must be 64, 128 or 256");
@@ -120,98 +106,118 @@ Tensor umma_rate(int64_t mode, int64_t n, int64_t reps, int64_t alt, int64_t cta
   return out;
 }
 
-// Hop mode (memory = "ring"): kv_buf holds ONE owner's slot ([1, 2, b*hk, n_k, d]); the launch visits that owner only
-// and carries the online-softmax state (un-normalised O, running max / sum) in fp32 buffers between launches.
-struct FwdHop {
-  int owner = -1;        // -1: single-launch mode
-  int world = 0;
-  float* carry_o = nullptr;
-  float* carry_ml = nullptr;
-  bool carry_in = false, carry_out = false;
-};
+// ---------------------------------------------------------------------------------------------
+// the attention problem: every attention op ends with these arguments, in this order
+// (ops/fused.py:AttnProblem.tail produces them)
+// ---------------------------------------------------------------------------------------------
+#define PROBLEM_SCHEMA                                                                                               \
+  "Tensor? kmask_bits, int batch, int heads, int kv_heads, int rank, bool causal, int window, float scale, float " \
+  "softclamp, int pos_stride, int seg_len, int[] base0, int[] base1, int q_pos_offset, int[] hop_owner"
+#define PROBLEM_PARAMS                                                                                               \
+  const c10::optional<Tensor>& kmask_bits, int64_t batch, int64_t heads, int64_t kv_heads, int64_t rank, bool causal, \
+      int64_t window, double scale, double softclamp, int64_t pos_stride, int64_t seg_len, at::IntArrayRef base0,  \
+      at::IntArrayRef base1, int64_t q_pos_offset, at::IntArrayRef hop_owner
+#define PROBLEM_ARGS                                                                                              \
+  kmask_bits, batch, heads, kv_heads, rank, causal, window, scale, softclamp, pos_stride, seg_len, base0, base1, \
+      q_pos_offset, hop_owner
 
-std::tuple<Tensor, Tensor> attn_fwd_impl(const Tensor& q, const Tensor& kv_buf, at::IntArrayRef peer_ptrs,
-                                         const c10::optional<Tensor>& ready_opt,
-                                         const c10::optional<Tensor>& kmask_bits, int64_t kv_heads, int64_t rank,
-                                         bool causal, int64_t window, double scale, double softclamp,
-                                         int64_t pos_stride, int64_t seg_len, at::IntArrayRef base0,
-                                         at::IntArrayRef base1, int64_t q_pos_offset, at::IntArrayRef hop_owner,
-                                         const FwdHop& hop) {
-  check_16bit(q, "q");
+// Fills `p` from the problem arguments and the K/V buffer kv_buf [slots][2][b*hk][n_k][d] (16 bit).  The ring size is
+// the length of the position map.  The buffer holds either every owner's slot, and then hop 0 is this rank, or one
+// owner's slot only (memory = "ring": one launch per hop), and then the launch visits exactly that owner.
+void parse_problem(rab::AttnProblem& p, const Tensor& kv_buf, int n_q, PROBLEM_PARAMS) {
   check_16bit(kv_buf, "kv_buf");
-  const bool hop_mode = hop.owner >= 0;
-  TORCH_CHECK(q.dim() == 4 && q.is_contiguous(), "q must be contiguous [b, n, h, d]");
-  TORCH_CHECK(kv_buf.dim() == 5 && kv_buf.is_contiguous(), "kv_buf must be contiguous [world, 2, b*hk, n_k, d]");
-  TORCH_CHECK(kv_buf.scalar_type() == q.scalar_type());
-  const int b = q.size(0), n_q = q.size(1), h = q.size(2), d = q.size(3);
-  const int world = hop_mode ? hop.world : (int)kv_buf.size(0), n_k = kv_buf.size(3);
-  TORCH_CHECK(kv_buf.size(1) == 2 && kv_buf.size(2) == b * kv_heads && kv_buf.size(4) == d);
-  TORCH_CHECK(d == 64 || d == 128, "head dim must be 64 or 128");
-  TORCH_CHECK(h % kv_heads == 0);
-  TORCH_CHECK(world <= rab::kMaxWorld);
-  if (hop_mode) {
-    TORCH_CHECK(kv_buf.size(0) == 1 && hop.owner < world && hop_owner.size() == 1 && hop_owner[0] == hop.owner);
+  TORCH_CHECK(kv_buf.dim() == 5 && kv_buf.is_contiguous(), "kv_buf must be contiguous [slots, 2, b*hk, n_k, d]");
+  TORCH_CHECK(kv_buf.size(1) == 2 && kv_buf.size(2) == batch * kv_heads);
+  TORCH_CHECK(kv_buf.size(4) == 64 || kv_buf.size(4) == 128, "head dim must be 64 or 128");
+  TORCH_CHECK(heads % kv_heads == 0);
+  const int world = (int)base0.size(), slots = (int)kv_buf.size(0);
+  TORCH_CHECK(world >= 1 && world <= rab::kMaxWorld && (int)base1.size() == world,
+              "position map needs one base per rank, at most ", rab::kMaxWorld);
+  TORCH_CHECK(rank >= 0 && rank < world);
+  TORCH_CHECK(hop_owner.size() >= 1 && (int)hop_owner.size() <= world);
+  for (int64_t o : hop_owner) TORCH_CHECK(o >= 0 && o < world, "hop owner out of range");
+  if (slots == world) {
+    TORCH_CHECK(hop_owner[0] == rank, "hop 0 must be this rank");
   } else {
-    TORCH_CHECK((int)peer_ptrs.size() == world && ready_opt.has_value());
-    TORCH_CHECK(ready_opt->is_cuda() && ready_opt->scalar_type() == at::kInt && ready_opt->numel() >= world);
-    TORCH_CHECK(hop_owner.size() >= 1 && (int)hop_owner.size() <= world && hop_owner[0] == rank);
+    TORCH_CHECK(slots == 1 && hop_owner.size() == 1, "a one-slot K/V buffer serves exactly one hop");
   }
-  c10::cuda::CUDAGuard guard(q.device());
-  auto stream = at::cuda::getCurrentCUDAStream();
-
-  Tensor o = torch::empty_like(q);
-  Tensor lse = torch::empty({b, h, n_q}, q.options().dtype(at::kFloat));
-
-  rab::AttnFwdParams p;
-  std::memset(&p, 0, sizeof(p));
-  p.batch = b; p.heads = h; p.kv_heads = (int)kv_heads;
-  p.n_q = n_q; p.n_k = n_k; p.world = world; p.rank = (int)rank;
+  p.batch = (int)batch; p.heads = (int)heads; p.kv_heads = (int)kv_heads;
+  p.n_q = n_q; p.n_k = (int)kv_buf.size(3);
+  p.world = world; p.rank = (int)rank;
   p.causal = causal; p.window = (int)window;
-  p.is_bf16 = q.scalar_type() == at::kBFloat16;
+  p.is_bf16 = kv_buf.scalar_type() == at::kBFloat16;
   p.scale = (float)scale; p.softclamp = (float)softclamp;
-  fill_posmap(p.pos, pos_stride, seg_len, base0, base1, world);
+  p.pos.stride = (int)pos_stride;
+  p.pos.seg_len = (int)seg_len;
+  for (int i = 0; i < world; ++i) {
+    p.pos.base0[i] = (int)base0[i];
+    p.pos.base1[i] = (int)base1[i];
+  }
   p.q_pos_offset = (int)q_pos_offset;
   p.hop_count = (int)hop_owner.size();
   for (int i = 0; i < p.hop_count; ++i) p.hop_owner[i] = (int)hop_owner[i];
-  p.o = o.data_ptr();
-  p.lse = lse.data_ptr<float>();
   if (kmask_bits.has_value()) {
     const Tensor& km = *kmask_bits;
     TORCH_CHECK(km.is_cuda() && km.scalar_type() == at::kInt && km.is_contiguous() && km.dim() == 3);
-    TORCH_CHECK(km.size(0) == world && km.size(1) == b && km.size(2) % 4 == 0 && km.size(2) * 32 >= n_k);
+    TORCH_CHECK(km.size(0) == world && km.size(1) == batch && km.size(2) % 4 == 0 && km.size(2) * 32 >= p.n_k);
     p.kmask_bits = reinterpret_cast<const uint32_t*>(km.data_ptr<int>());
     p.kmask_words = km.size(2);
   }
-  p.slot_bytes = 2ull * b * kv_heads * n_k * d * 2;
-  // the kernels address owner o's K / V at slot o of the buffer; in hop mode the one slot we were given IS slot
-  // `owner`, so the base is shifted down by owner slots (only that slot is ever dereferenced)
-  uint8_t* kv_base = reinterpret_cast<uint8_t*>(kv_buf.data_ptr()) - (hop_mode ? hop.owner * p.slot_bytes : 0);
-  p.kv_local = kv_base;
-  if (hop_mode) {
-    p.all_ready = 1;
-    p.carry_o = hop.carry_o;
-    p.carry_ml = hop.carry_ml;
-    p.carry_in = hop.carry_in;
-    p.carry_out = hop.carry_out;
-  } else {
-    for (int i = 0; i < world; ++i)
-      p.kv_peer[i] = peer_ptrs[i] ? reinterpret_cast<const uint8_t*>(peer_ptrs[i]) : p.kv_local + i * p.slot_bytes;
-    p.ready = reinterpret_cast<uint32_t*>(ready_opt->data_ptr<int>());
-    rab::cuda_check(cudaMemsetAsync(p.ready, 0, sizeof(uint32_t) * world, stream), "ready memset");
-    p.fetch_times = (g_fetch_times != nullptr && g_fetch_times_rows >= sm_count()) ? g_fetch_times : nullptr;
-  }
+}
 
+// Address of owner slot 0 as the kernels see it.  They address owner o's K / V at slot o; a one-slot buffer IS slot
+// hop_owner[0], so its base moves down by that many slots (only that slot is ever dereferenced).
+uint8_t* kv_slot0(const Tensor& kv_buf, const rab::AttnProblem& p) {
+  const size_t slot_bytes = kv_buf.nbytes() / kv_buf.size(0);
+  const int shift = kv_buf.size(0) == p.world ? 0 : p.hop_owner[0];
+  return reinterpret_cast<uint8_t*>(kv_buf.data_ptr()) - shift * slot_bytes;
+}
+
+// K/V of every owner, [world][2][b*hk][n_k][d] -> dims (d, n_k, b*hk, 2*world), box (64, 128, 1, 1)
+CUtensorMap make_kv_map(const Tensor& kv_buf, const rab::AttnProblem& p) {
+  const uint64_t d = kv_buf.size(4), rows = (uint64_t)p.batch * p.kv_heads;
+  uint64_t dims[4] = {d, (uint64_t)p.n_k, rows, (uint64_t)2 * p.world};
+  uint64_t str[3] = {d * 2, (uint64_t)p.n_k * d * 2, rows * p.n_k * d * 2};
+  uint32_t box[4] = {64, 128, 1, 1};
+  return rab::make_tmap_bf16(kv_slot0(kv_buf, p), 4, dims, str, box, rab::TmapSwizzle::B128);
+}
+
+// per-owner ready flags: int32, one per ring rank (null when not given)
+uint32_t* ready_flags(const c10::optional<Tensor>& ready, int world) {
+  if (!ready.has_value()) return nullptr;
+  TORCH_CHECK(ready->is_cuda() && ready->scalar_type() == at::kInt && ready->numel() >= world,
+              "ready must be int32 [world] on the GPU");
+  return reinterpret_cast<uint32_t*>(ready->data_ptr<int>());
+}
+
+// ---------------------------------------------------------------------------------------------
+// fused ring attention forward
+// ---------------------------------------------------------------------------------------------
+void parse_fwd(rab::AttnFwdParams& p, const Tensor& q, const Tensor& kv_buf, PROBLEM_PARAMS) {
+  check_16bit(q, "q");
+  TORCH_CHECK(q.dim() == 4 && q.is_contiguous(), "q must be contiguous [b, n, h, d]");
+  std::memset(&p, 0, sizeof(p));
+  parse_problem(p, kv_buf, (int)q.size(1), PROBLEM_ARGS);
+  TORCH_CHECK(kv_buf.scalar_type() == q.scalar_type());
+  TORCH_CHECK(q.size(0) == batch && q.size(2) == heads && q.size(3) == kv_buf.size(4));
+  p.slot_bytes = kv_buf.nbytes() / kv_buf.size(0);
+  p.kv_local = kv_slot0(kv_buf, p);
+}
+
+std::tuple<Tensor, Tensor> launch_fwd(const Tensor& q, const Tensor& kv_buf, rab::AttnFwdParams& p) {
+  c10::cuda::CUDAGuard guard(q.device());
+  const int b = p.batch, n_q = p.n_q, h = p.heads, d = q.size(3);
+  Tensor o = torch::empty_like(q);
+  Tensor lse = torch::empty({b, h, n_q}, q.options().dtype(at::kFloat));
+  p.o = o.data_ptr();
+  p.lse = lse.data_ptr<float>();
   // Q: [b, n, h, d] -> dims (d, h, n, b), box (64, 1, 128, 1)
   uint64_t qdims[4] = {(uint64_t)d, (uint64_t)h, (uint64_t)n_q, (uint64_t)b};
   uint64_t qstr[3] = {(uint64_t)d * 2, (uint64_t)h * d * 2, (uint64_t)n_q * h * d * 2};
   uint32_t qbox[4] = {64, 1, 128, 1};
   CUtensorMap map_q = rab::make_tmap_bf16(q.data_ptr(), 4, qdims, qstr, qbox, rab::TmapSwizzle::B128);
-  // KV: [world, 2, b*hk, n_k, d] -> dims (d, n_k, b*hk, 2*world), box (64, 128, 1, 1)
-  uint64_t kdims[4] = {(uint64_t)d, (uint64_t)n_k, (uint64_t)b * kv_heads, (uint64_t)2 * world};
-  uint64_t kstr[3] = {(uint64_t)d * 2, (uint64_t)n_k * d * 2, (uint64_t)b * kv_heads * n_k * d * 2};
-  uint32_t kbox[4] = {64, 128, 1, 1};
-  CUtensorMap map_kv = rab::make_tmap_bf16(kv_base, 4, kdims, kstr, kbox, rab::TmapSwizzle::B128);
-
+  CUtensorMap map_kv = make_kv_map(kv_buf, p);
+  auto stream = at::cuda::getCurrentCUDAStream();
   if (d == 128) {
     rab::launch_attn_fwd<128>(map_q, map_kv, p, sm_count(), stream);
   } else {
@@ -220,42 +226,43 @@ std::tuple<Tensor, Tensor> attn_fwd_impl(const Tensor& q, const Tensor& kv_buf, 
   return {o, lse};
 }
 
+// The whole ring in one launch: kv_buf [world, 2, b*hk, n_k, d] holds this rank's slot; the kernel's fetchers pull
+// owner o's slot from peer_ptrs[o] (0: already local) and publish it through the ready flags.
 std::tuple<Tensor, Tensor> attn_fwd(const Tensor& q, const Tensor& kv_buf, at::IntArrayRef peer_ptrs,
-                                    const Tensor& ready, const c10::optional<Tensor>& kmask_bits,
-                                    int64_t kv_heads, int64_t rank, bool causal, int64_t window, double scale,
-                                    double softclamp, int64_t pos_stride, int64_t seg_len, at::IntArrayRef base0,
-                                    at::IntArrayRef base1, int64_t q_pos_offset, at::IntArrayRef hop_owner) {
-  return attn_fwd_impl(q, kv_buf, peer_ptrs, ready, kmask_bits, kv_heads, rank, causal, window, scale, softclamp,
-                       pos_stride, seg_len, base0, base1, q_pos_offset, hop_owner, FwdHop{});
+                                    const Tensor& ready, PROBLEM_PARAMS) {
+  rab::AttnFwdParams p;
+  parse_fwd(p, q, kv_buf, PROBLEM_ARGS);
+  TORCH_CHECK(kv_buf.size(0) == p.world && (int)peer_ptrs.size() == p.world, "attn_fwd needs every owner's slot");
+  for (int i = 0; i < p.world; ++i)
+    p.kv_peer[i] = peer_ptrs[i] ? reinterpret_cast<const uint8_t*>(peer_ptrs[i]) : p.kv_local + i * p.slot_bytes;
+  p.ready = ready_flags(ready, p.world);
+  c10::cuda::CUDAGuard guard(q.device());
+  rab::cuda_check(cudaMemsetAsync(p.ready, 0, sizeof(uint32_t) * p.world, at::cuda::getCurrentCUDAStream()),
+                  "ready memset");
+  p.fetch_times = (g_fetch_times != nullptr && g_fetch_times_rows >= sm_count()) ? g_fetch_times : nullptr;
+  return launch_fwd(q, kv_buf, p);
 }
 
-// One ring hop of the forward: q against owner `owner`'s K / V slot.  carry_o fp32 [b, n_q, h, d] and carry_ml fp32
-// [2, b*h, n_q] hold the online-softmax state between hops; the launch with carry_out = false writes the final O / lse.
-std::tuple<Tensor, Tensor> attn_fwd_hop(const Tensor& q, const Tensor& kv_slot, int64_t owner, int64_t world,
-                                        Tensor carry_o, Tensor carry_ml, bool carry_in, bool carry_out,
-                                        const c10::optional<Tensor>& kmask_bits, int64_t kv_heads, int64_t rank,
-                                        bool causal, int64_t window, double scale, double softclamp,
-                                        int64_t pos_stride, int64_t seg_len, at::IntArrayRef base0,
-                                        at::IntArrayRef base1, int64_t q_pos_offset) {
-  TORCH_CHECK(q.dim() == 4);
-  const int64_t b = q.size(0), n_q = q.size(1), h = q.size(2), d = q.size(3);
+// One ring hop of the forward: q against the one owner slot kv_slot [1, 2, b*hk, n_k, d] of owner hop_owner[0].
+// carry_o fp32 [b, n_q, h, d] and carry_ml fp32 [2, b*h, n_q] hold the online-softmax state between hops; the launch
+// with carry_out = false writes the final O / lse.
+std::tuple<Tensor, Tensor> attn_fwd_hop(const Tensor& q, const Tensor& kv_slot, Tensor carry_o, Tensor carry_ml,
+                                        bool carry_in, bool carry_out, PROBLEM_PARAMS) {
+  rab::AttnFwdParams p;
+  parse_fwd(p, q, kv_slot, PROBLEM_ARGS);
+  TORCH_CHECK(kv_slot.size(0) == 1, "attn_fwd_hop takes one owner's slot");
+  const int64_t b = p.batch, n_q = p.n_q, h = p.heads, d = q.size(3);
   TORCH_CHECK(carry_o.is_cuda() && carry_o.scalar_type() == at::kFloat && carry_o.is_contiguous() &&
               carry_o.numel() == b * n_q * h * d, "carry_o must be fp32 [b, n_q, h, d]");
   TORCH_CHECK(carry_ml.is_cuda() && carry_ml.scalar_type() == at::kFloat && carry_ml.is_contiguous() &&
               carry_ml.numel() == 2 * b * h * n_q, "carry_ml must be fp32 [2, b*h, n_q]");
-  TORCH_CHECK(owner >= 0 && owner < world);
-  FwdHop hop;
-  hop.owner = (int)owner;
-  hop.world = (int)world;
-  hop.carry_o = carry_o.data_ptr<float>();
-  hop.carry_ml = carry_ml.data_ptr<float>();
-  hop.carry_in = carry_in;
-  hop.carry_out = carry_out;
-  const int64_t owners[1] = {owner};
-  return attn_fwd_impl(q, kv_slot, {}, c10::nullopt, kmask_bits, kv_heads, rank, causal, window, scale, softclamp,
-                       pos_stride, seg_len, base0, base1, q_pos_offset, at::IntArrayRef(owners, 1), hop);
+  p.all_ready = 1;
+  p.carry_o = carry_o.data_ptr<float>();
+  p.carry_ml = carry_ml.data_ptr<float>();
+  p.carry_in = carry_in;
+  p.carry_out = carry_out;
+  return launch_fwd(q, kv_slot, p);
 }
-
 
 // ---------------------------------------------------------------------------------------------
 // fused ring attention backward
@@ -283,70 +290,39 @@ struct BwdSetup {
   CUtensorMap map_qd128, map_qd64, map_kv;
 };
 
+// the two-kernel backward: qdo_buf [world][2][b*h][n_q][d], kv_buf [world][2][b*hk][n_k][d], stat_buf
+// [world][2][b*h][n_pad], all gathered
 BwdSetup make_bwd_setup(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
-                        const c10::optional<Tensor>& ready, int64_t ready_target,
-                        const c10::optional<Tensor>& kmask_bits, int64_t batch, int64_t heads, int64_t kv_heads,
-                        int64_t rank, bool causal, int64_t window, double scale, double softclamp, int64_t pos_stride,
-                        int64_t seg_len, at::IntArrayRef base0, at::IntArrayRef base1, int64_t q_pos_offset,
-                        at::IntArrayRef hop_owner) {
+                        const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
   check_16bit(qdo_buf, "qdo_buf");
-  check_16bit(kv_buf, "kv_buf");
-  TORCH_CHECK(qdo_buf.is_contiguous() && kv_buf.is_contiguous() && stat_buf.is_contiguous());
-  TORCH_CHECK(qdo_buf.dim() == 5 && kv_buf.dim() == 5 && stat_buf.dim() == 4);
-  const int world = kv_buf.size(0), n_k = kv_buf.size(3), d = kv_buf.size(4);
-  const int n_q = qdo_buf.size(3);
-  TORCH_CHECK(qdo_buf.size(0) == world && qdo_buf.size(2) == batch * heads && qdo_buf.size(4) == d);
-  TORCH_CHECK(kv_buf.size(2) == batch * kv_heads && stat_buf.size(0) == world && stat_buf.size(2) == batch * heads);
-  TORCH_CHECK(d == 64 || d == 128);
-  TORCH_CHECK(hop_owner.size() >= 1 && (int)hop_owner.size() <= world && hop_owner[0] == rank);
+  TORCH_CHECK(qdo_buf.is_contiguous() && stat_buf.is_contiguous());
+  TORCH_CHECK(qdo_buf.dim() == 5 && stat_buf.dim() == 4);
   BwdSetup s;
   rab::AttnBwdParams& p = s.p;
   std::memset(&p, 0, sizeof(p));
-  p.batch = (int)batch; p.heads = (int)heads; p.kv_heads = (int)kv_heads;
-  p.n_q = n_q; p.n_k = n_k; p.n_pad = stat_buf.size(3);
-  p.world = world; p.rank = (int)rank;
-  p.causal = causal; p.window = (int)window;
-  p.is_bf16 = kv_buf.scalar_type() == at::kBFloat16;
-  p.scale = (float)scale; p.softclamp = (float)softclamp;
-  fill_posmap(p.pos, pos_stride, seg_len, base0, base1, world);
-  p.q_pos_offset = (int)q_pos_offset;
-  p.hop_count = (int)hop_owner.size();
-  for (int i = 0; i < p.hop_count; ++i) p.hop_owner[i] = (int)hop_owner[i];
+  parse_problem(p, kv_buf, (int)qdo_buf.size(3), PROBLEM_ARGS);
+  const int world = p.world, n_q = p.n_q, d = kv_buf.size(4);
+  TORCH_CHECK(kv_buf.size(0) == world, "the two-kernel backward needs every owner's slot");
+  TORCH_CHECK(qdo_buf.size(0) == world && qdo_buf.size(2) == batch * heads && qdo_buf.size(4) == d);
+  TORCH_CHECK(stat_buf.size(0) == world && stat_buf.size(2) == batch * heads);
+  p.n_pad = stat_buf.size(3);
   p.stat = stat_buf.data_ptr<float>();
-  if (kmask_bits.has_value()) {
-    const Tensor& km = *kmask_bits;
-    TORCH_CHECK(km.is_cuda() && km.scalar_type() == at::kInt && km.is_contiguous() && km.dim() == 3);
-    TORCH_CHECK(km.size(0) == world && km.size(1) == batch && km.size(2) % 4 == 0 && km.size(2) * 32 >= n_k);
-    p.kmask_bits = reinterpret_cast<const uint32_t*>(km.data_ptr<int>());
-    p.kmask_words = km.size(2);
-  }
-  if (ready.has_value()) {
-    TORCH_CHECK(ready->is_cuda() && ready->scalar_type() == at::kInt && ready->numel() >= world);
-    p.ready = reinterpret_cast<const uint32_t*>(ready->data_ptr<int>());
-    p.ready_target = (uint32_t)ready_target;
-  }
+  p.ready = ready_flags(ready, world);
+  p.ready_target = p.ready ? (uint32_t)ready_target : 0;
   uint64_t qdims[4] = {(uint64_t)d, (uint64_t)n_q, (uint64_t)batch * heads, (uint64_t)2 * world};
   uint64_t qstr[3] = {(uint64_t)d * 2, (uint64_t)n_q * d * 2, (uint64_t)batch * heads * n_q * d * 2};
   uint32_t qbox128[4] = {64, 128, 1, 1};
   uint32_t qbox64[4] = {64, 64, 1, 1};
   s.map_qd128 = rab::make_tmap_bf16(qdo_buf.data_ptr(), 4, qdims, qstr, qbox128, rab::TmapSwizzle::B128);
   s.map_qd64 = rab::make_tmap_bf16(qdo_buf.data_ptr(), 4, qdims, qstr, qbox64, rab::TmapSwizzle::B128);
-  uint64_t kdims[4] = {(uint64_t)d, (uint64_t)n_k, (uint64_t)batch * kv_heads, (uint64_t)2 * world};
-  uint64_t kstr[3] = {(uint64_t)d * 2, (uint64_t)n_k * d * 2, (uint64_t)batch * kv_heads * n_k * d * 2};
-  uint32_t kbox[4] = {64, 128, 1, 1};
-  s.map_kv = rab::make_tmap_bf16(kv_buf.data_ptr(), 4, kdims, kstr, kbox, rab::TmapSwizzle::B128);
+  s.map_kv = make_kv_map(kv_buf, p);
   return s;
 }
 
 Tensor attn_bwd_dq(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
-                   const c10::optional<Tensor>& ready, int64_t ready_target, const c10::optional<Tensor>& kmask_bits,
-                   int64_t batch, int64_t heads, int64_t kv_heads, int64_t rank, bool causal, int64_t window,
-                   double scale, double softclamp, int64_t pos_stride, int64_t seg_len, at::IntArrayRef base0,
-                   at::IntArrayRef base1, int64_t q_pos_offset, at::IntArrayRef hop_owner) {
+                   const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
   c10::cuda::CUDAGuard guard(kv_buf.device());
-  BwdSetup s = make_bwd_setup(qdo_buf, kv_buf, stat_buf, ready, ready_target, kmask_bits, batch, heads, kv_heads, rank,
-                              causal, window, scale, softclamp, pos_stride, seg_len, base0, base1, q_pos_offset,
-                              hop_owner);
+  BwdSetup s = make_bwd_setup(qdo_buf, kv_buf, stat_buf, ready, ready_target, PROBLEM_ARGS);
   const int d = kv_buf.size(4);
   Tensor dq = torch::empty({batch, s.p.n_q, heads, d}, kv_buf.options());
   s.p.dq = dq.data_ptr();
@@ -360,15 +336,9 @@ Tensor attn_bwd_dq(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& st
 }
 
 std::tuple<Tensor, Tensor> attn_bwd_dkdv(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
-                                         const c10::optional<Tensor>& ready, int64_t ready_target,
-                                         const c10::optional<Tensor>& kmask_bits, int64_t batch, int64_t heads,
-                                         int64_t kv_heads, int64_t rank, bool causal, int64_t window, double scale,
-                                         double softclamp, int64_t pos_stride, int64_t seg_len, at::IntArrayRef base0,
-                                         at::IntArrayRef base1, int64_t q_pos_offset, at::IntArrayRef hop_owner) {
+                                         const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
   c10::cuda::CUDAGuard guard(kv_buf.device());
-  BwdSetup s = make_bwd_setup(qdo_buf, kv_buf, stat_buf, ready, ready_target, kmask_bits, batch, heads, kv_heads, rank,
-                              causal, window, scale, softclamp, pos_stride, seg_len, base0, base1, q_pos_offset,
-                              hop_owner);
+  BwdSetup s = make_bwd_setup(qdo_buf, kv_buf, stat_buf, ready, ready_target, PROBLEM_ARGS);
   const int d = kv_buf.size(4);
   Tensor dk = torch::empty({batch, s.p.n_k, kv_heads, d}, kv_buf.options());
   Tensor dv = torch::empty({batch, s.p.n_k, kv_heads, d}, kv_buf.options());
@@ -385,81 +355,43 @@ std::tuple<Tensor, Tensor> attn_bwd_dkdv(const Tensor& qdo_buf, const Tensor& kv
 
 // One-kernel (5-GEMM) ring backward, head dim 128 (attn_bwd_fused_sm100.cu).
 //   qdo [2][b*h][n_q][d] 16 bit and stat [2][b*h][n_pad] fp32: this rank's bwd_prep output
-//   kv_buf [world][2][b*hk][n_k][d]: the K/V gather (slot o valid once ready[o] >= ready_target; no flags: all valid)
+//   kv_buf: the K/V gather [world][2][b*hk][n_k][d] (slot o valid once ready[o] >= ready_target; no flags: all valid),
+//           or one owner's slot [1][2][b*hk][n_k][d] (memory = "ring": one launch per hop)
 //   dq_acc fp32 [b*h][n_pad][d], zeroed by the caller: dQ (unscaled) is ADDED into it
 //   dkv_acc_ptrs: empty -> dK, dV are returned as 16 bit [b, n_k, hk, d] (single rank);
 //                 else one pointer per ring rank to that rank's zeroed fp32 [2][b*hk][nk_pad][d] accumulator (peer
-//                 mapped): the kernel adds its dK / dV tiles into the owner's accumulator and returns empty tensors
+//                 mapped): the kernel adds its dK / dV tiles into the owner's accumulator and returns empty tensors.
+// dq_acc and the dK / dV accumulators keep adding up across the per-hop launches.
 std::tuple<Tensor, Tensor> attn_bwd_ring(const Tensor& qdo, const Tensor& kv_buf, const Tensor& stat, Tensor dq_acc,
                                          const c10::optional<Tensor>& ready, int64_t ready_target,
-                                         const c10::optional<Tensor>& kmask_bits, int64_t batch, int64_t heads,
-                                         int64_t kv_heads, int64_t rank, bool causal, int64_t window, double scale,
-                                         double softclamp, int64_t pos_stride, int64_t seg_len, at::IntArrayRef base0,
-                                         at::IntArrayRef base1, int64_t q_pos_offset, at::IntArrayRef hop_owner,
-                                         at::IntArrayRef dkv_acc_ptrs, int64_t nk_pad, int64_t world_size,
-                                         int64_t slot_owner) {
-  // slot_owner >= 0 (memory = "ring"): kv_buf is ONE owner's slot [1, 2, b*hk, n_k, d] of a `world_size` ring and
-  // hop_owner == [slot_owner]; dq_acc and the dK / dV accumulators keep adding up across the per-hop launches
+                                         at::IntArrayRef dkv_acc_ptrs, int64_t nk_pad, PROBLEM_PARAMS) {
   check_16bit(qdo, "qdo");
-  check_16bit(kv_buf, "kv_buf");
-  TORCH_CHECK(qdo.is_contiguous() && kv_buf.is_contiguous() && stat.is_contiguous() && dq_acc.is_contiguous());
-  TORCH_CHECK(kv_buf.dim() == 5 && qdo.dim() == 4 && stat.dim() == 3 && dq_acc.dim() == 3);
-  const bool hop_mode = slot_owner >= 0;
-  const int world = hop_mode ? (int)world_size : (int)kv_buf.size(0), n_k = kv_buf.size(3), d = kv_buf.size(4);
-  const int n_q = qdo.size(2), n_pad = stat.size(2);
+  TORCH_CHECK(qdo.is_contiguous() && stat.is_contiguous() && dq_acc.is_contiguous());
+  TORCH_CHECK(qdo.dim() == 4 && stat.dim() == 3 && dq_acc.dim() == 3);
+  rab::AttnBwdFusedParams p;
+  std::memset(&p, 0, sizeof(p));
+  parse_problem(p, kv_buf, (int)qdo.size(2), PROBLEM_ARGS);
+  const int world = p.world, n_q = p.n_q, n_k = p.n_k, n_pad = stat.size(2), d = kv_buf.size(4);
   TORCH_CHECK(d == 128, "attn_bwd_ring: head dim 128 only");
   TORCH_CHECK(qdo.size(0) == 2 && qdo.size(1) == batch * heads && qdo.size(3) == d);
   TORCH_CHECK(stat.size(0) == 2 && stat.size(1) == batch * heads && stat.scalar_type() == at::kFloat);
   TORCH_CHECK(n_pad % 64 == 0 && n_pad >= n_q);
   TORCH_CHECK(dq_acc.scalar_type() == at::kFloat && dq_acc.size(0) == batch * heads && dq_acc.size(1) == n_pad &&
               dq_acc.size(2) == d);
-  TORCH_CHECK(kv_buf.size(1) == 2 && kv_buf.size(2) == batch * kv_heads && heads % kv_heads == 0);
-  TORCH_CHECK(world <= rab::kMaxWorld && hop_owner.size() >= 1 && (int)hop_owner.size() <= world);
-  if (hop_mode) {
-    TORCH_CHECK(kv_buf.size(0) == 1 && slot_owner < world && hop_owner.size() == 1 && hop_owner[0] == slot_owner);
-  } else {
-    TORCH_CHECK(hop_owner[0] == rank);
-  }
   c10::cuda::CUDAGuard guard(kv_buf.device());
   auto stream = at::cuda::getCurrentCUDAStream();
 
-  rab::AttnBwdFusedParams p;
-  std::memset(&p, 0, sizeof(p));
-  p.batch = (int)batch; p.heads = (int)heads; p.kv_heads = (int)kv_heads;
-  p.n_q = n_q; p.n_k = n_k; p.n_pad = n_pad; p.nk_pad = (int)nk_pad;
-  p.world = world; p.rank = (int)rank;
-  p.causal = causal; p.window = (int)window;
-  p.is_bf16 = kv_buf.scalar_type() == at::kBFloat16;
-  p.scale = (float)scale; p.softclamp = (float)softclamp;
-  fill_posmap(p.pos, pos_stride, seg_len, base0, base1, world);
-  p.q_pos_offset = (int)q_pos_offset;
-  p.hop_count = (int)hop_owner.size();
-  for (int i = 0; i < p.hop_count; ++i) p.hop_owner[i] = (int)hop_owner[i];
+  p.n_pad = n_pad; p.nk_pad = (int)nk_pad;
   p.self_owner[0] = (int)rank;
   p.stat = stat.data_ptr<float>();
-  if (kmask_bits.has_value()) {
-    const Tensor& km = *kmask_bits;
-    TORCH_CHECK(km.is_cuda() && km.scalar_type() == at::kInt && km.is_contiguous() && km.dim() == 3);
-    TORCH_CHECK(km.size(0) == world && km.size(1) == batch && km.size(2) % 4 == 0 && km.size(2) * 32 >= n_k);
-    p.kmask_bits = reinterpret_cast<const uint32_t*>(km.data_ptr<int>());
-    p.kmask_words = km.size(2);
-  }
-  if (ready.has_value()) {
-    TORCH_CHECK(ready->is_cuda() && ready->scalar_type() == at::kInt && ready->numel() >= world);
-    p.ready = reinterpret_cast<const uint32_t*>(ready->data_ptr<int>());
-    p.ready_target = (uint32_t)ready_target;
-  }
+  p.ready = ready_flags(ready, world);
+  p.ready_target = p.ready ? (uint32_t)ready_target : 0;
   // local Q / dO: dims (d, n_q, b*h, 2), box (64, 64, 1, 1)
   uint64_t qdims[4] = {(uint64_t)d, (uint64_t)n_q, (uint64_t)batch * heads, 2};
   uint64_t qstr[3] = {(uint64_t)d * 2, (uint64_t)n_q * d * 2, (uint64_t)batch * heads * n_q * d * 2};
   uint32_t qbox64[4] = {64, 64, 1, 1};
   CUtensorMap map_qd64 = rab::make_tmap_bf16(qdo.data_ptr(), 4, qdims, qstr, qbox64, rab::TmapSwizzle::B128);
-  uint64_t kdims[4] = {(uint64_t)d, (uint64_t)n_k, (uint64_t)batch * kv_heads, (uint64_t)2 * world};
-  uint64_t kstr[3] = {(uint64_t)d * 2, (uint64_t)n_k * d * 2, (uint64_t)batch * kv_heads * n_k * d * 2};
-  uint32_t kbox[4] = {64, 128, 1, 1};
-  const uint8_t* kv_base = reinterpret_cast<const uint8_t*>(kv_buf.data_ptr()) -
-                           (hop_mode ? (size_t)slot_owner * kstr[2] * 2 : 0);  // see attn_fwd_impl
-  CUtensorMap map_kv = rab::make_tmap_bf16(kv_base, 4, kdims, kstr, kbox, rab::TmapSwizzle::B128);
+  CUtensorMap map_kv = make_kv_map(kv_buf, p);
   // dQ accumulator: 2-D (d, b*h*n_pad) fp32, box 32 columns x 32 rows, no swizzle (rows written lane-contiguous)
   uint64_t adims[2] = {(uint64_t)d, (uint64_t)batch * heads * n_pad};
   uint64_t astr[1] = {(uint64_t)d * 4};
@@ -706,9 +638,9 @@ TORCH_LIBRARY(rab, m) {
   m.def("umma_rate(int mode, int n, int reps, int alt, int ctas) -> Tensor");
   m.def("umma_probe(Tensor a, Tensor b, int mode, int n, int k, int idesc, int a_lbo, int a_sbo, int b_lbo, int "
         "b_sbo, int b_kstep) -> Tensor");
-  m.def("attn_fwd(Tensor q, Tensor kv_buf, int[] peer_ptrs, Tensor ready, Tensor? kmask_bits, int kv_heads, int rank, "
-        "bool causal, int window, float scale, float softclamp, int pos_stride, int seg_len, int[] base0, int[] "
-        "base1, int q_pos_offset, int[] hop_owner) -> (Tensor, Tensor)");
+  m.def("attn_fwd(Tensor q, Tensor kv_buf, int[] peer_ptrs, Tensor ready, " PROBLEM_SCHEMA ") -> (Tensor, Tensor)");
+  m.def("attn_fwd_hop(Tensor q, Tensor kv_slot, Tensor(a!) carry_o, Tensor(b!) carry_ml, bool carry_in, bool carry_out, "
+        PROBLEM_SCHEMA ") -> (Tensor, Tensor)");
   m.def("pack_kv(Tensor k, Tensor v, Tensor(a!) slot, int which=3) -> ()");
   m.def("rotary(Tensor x, Tensor angles, Tensor(a!) out, bool head_major, float sign) -> ()");
   m.def("tree_decode(Tensor q, Tensor? k, Tensor? v, Tensor? k_scale, Tensor? v_scale, Tensor(a!) scratch, Tensor(b!) "
@@ -717,20 +649,12 @@ TORCH_LIBRARY(rab, m) {
         "int grid, bool tensor_core) -> ()");
   m.def("tree_decode_max_ctas(int d, int kv_kind, bool tensor_core) -> int");
   m.def("bwd_prep(Tensor q, Tensor o, Tensor dout, Tensor lse, Tensor(a!) qdo_buf, Tensor(b!) stat_buf, int rank) -> ()");
-  m.def("attn_bwd_dq(Tensor qdo_buf, Tensor kv_buf, Tensor stat_buf, Tensor? ready, int ready_target, Tensor? "
-        "kmask_bits, int batch, int heads, int kv_heads, int rank, bool causal, int window, float scale, float "
-        "softclamp, int pos_stride, int seg_len, int[] base0, int[] base1, int q_pos_offset, int[] hop_owner) -> Tensor");
-  m.def("attn_bwd_dkdv(Tensor qdo_buf, Tensor kv_buf, Tensor stat_buf, Tensor? ready, int ready_target, Tensor? "
-        "kmask_bits, int batch, int heads, int kv_heads, int rank, bool causal, int window, float scale, float "
-        "softclamp, int pos_stride, int seg_len, int[] base0, int[] base1, int q_pos_offset, int[] hop_owner) -> "
-        "(Tensor, Tensor)");
-  m.def("attn_bwd_ring(Tensor qdo, Tensor kv_buf, Tensor stat, Tensor(a!) dq_acc, Tensor? ready, int ready_target, "
-        "Tensor? kmask_bits, int batch, int heads, int kv_heads, int rank, bool causal, int window, float scale, float "
-        "softclamp, int pos_stride, int seg_len, int[] base0, int[] base1, int q_pos_offset, int[] hop_owner, int[] "
-        "dkv_acc_ptrs, int nk_pad, int world_size=0, int slot_owner=-1) -> (Tensor, Tensor)");
-  m.def("attn_fwd_hop(Tensor q, Tensor kv_slot, int owner, int world, Tensor(a!) carry_o, Tensor(b!) carry_ml, bool "
-        "carry_in, bool carry_out, Tensor? kmask_bits, int kv_heads, int rank, bool causal, int window, float scale, "
-        "float softclamp, int pos_stride, int seg_len, int[] base0, int[] base1, int q_pos_offset) -> (Tensor, Tensor)");
+  m.def("attn_bwd_dq(Tensor qdo_buf, Tensor kv_buf, Tensor stat_buf, Tensor? ready, int ready_target, " PROBLEM_SCHEMA
+        ") -> Tensor");
+  m.def("attn_bwd_dkdv(Tensor qdo_buf, Tensor kv_buf, Tensor stat_buf, Tensor? ready, int ready_target, " PROBLEM_SCHEMA
+        ") -> (Tensor, Tensor)");
+  m.def("attn_bwd_ring(Tensor qdo, Tensor kv_buf, Tensor stat, Tensor(a!) dq_acc, Tensor? ready, int ready_target, int[] "
+        "dkv_acc_ptrs, int nk_pad, " PROBLEM_SCHEMA ") -> (Tensor, Tensor)");
   m.def("acc_convert(Tensor acc, Tensor(a!) out, float scale) -> ()");
   m.def("set_fetch_timing(Tensor? times) -> ()");
   m.def("device_barrier(int[] pad_ptrs, int rank, int epoch) -> ()");

@@ -43,9 +43,9 @@ struct PosMap {
 };
 
 // ------------------------------------------------------------------------------------------------
-// fused ring flash-attention forward
+// the attention problem the forward and both backwards share (one ring rank's view of it)
 // ------------------------------------------------------------------------------------------------
-struct AttnFwdParams {
+struct AttnProblem {
   int batch, heads, kv_heads;
   int n_q;      // local query rows
   int n_k;      // keys per owner slot
@@ -59,13 +59,19 @@ struct AttnFwdParams {
   PosMap pos;
   int q_pos_offset;   // added to query positions (cross-attention causal alignment)
   int hop_count;
-  int hop_owner[kMaxWorld];  // hop 0 is this rank
-  // outputs
-  void* o;       // [b, n_q, h, d] 16-bit
-  float* lse;    // [b, h, n_q] natural-log lse (+inf for rows with no visible key)
+  int hop_owner[kMaxWorld];  // owners visited; hop 0 is this rank unless the launch covers one hop only
   // key-padding bits: [world][batch][kmask_words] uint32 (bit set = keep), may be null
   const uint32_t* kmask_bits;
   int kmask_words;
+};
+
+// ------------------------------------------------------------------------------------------------
+// fused ring flash-attention forward
+// ------------------------------------------------------------------------------------------------
+struct AttnFwdParams : AttnProblem {
+  // outputs
+  void* o;       // [b, n_q, h, d] 16-bit
+  float* lse;    // [b, h, n_q] natural-log lse (+inf for rows with no visible key)
   // in-kernel K/V gather over NVLink
   uint8_t* kv_local;                  // this rank's [world][2][b*hk][n_k][d] buffer
   const uint8_t* kv_peer[kMaxWorld];  // kv_peer[o]: owner o's own [2][b*hk][n_k][d] slot (peer-mapped)
@@ -94,22 +100,12 @@ size_t attn_fwd_smem_bytes(int head_dim);
 // locally, the other slots arrive over NVLink (copy engines on a side stream, or an earlier kernel) and
 // are published through the per-owner ready flags.
 // ------------------------------------------------------------------------------------------------
-struct AttnBwdParams {
-  int batch, heads, kv_heads;
-  int n_q, n_k, n_pad;
-  int world, rank;
-  int causal, window, is_bf16;
-  float scale, softclamp;
-  PosMap pos;
-  int q_pos_offset;
-  int hop_count;
-  int hop_owner[kMaxWorld];
+struct AttnBwdParams : AttnProblem {
+  int n_pad;
   const float* stat;           // gathered [world][2][b*h][n_pad]
   void* dq;                    // [b, n_q, h, d]
   void* dk;                    // [b, n_k, hk, d]
   void* dv;                    // [b, n_k, hk, d]
-  const uint32_t* kmask_bits;  // [world][batch][kmask_words]
-  int kmask_words;
   const uint32_t* ready;       // [world] flags: slot o usable once ready[o] >= ready_target (may be null)
   uint32_t ready_target;
 };
@@ -128,20 +124,10 @@ void launch_attn_bwd_dkdv(const CUtensorMap& map_qd64, const CUtensorMap& map_kv
 //   dK/dV  : ring_reduce == 0: 16 bit [b, n_k, hk, d] written directly (single rank)
 //            ring_reduce == 1: added into owner o's fp32 [2][b*hk][nk_pad][d] accumulator through map_dkv[o]
 // ------------------------------------------------------------------------------------------------
-struct AttnBwdFusedParams {
-  int batch, heads, kv_heads;
-  int n_q, n_k, n_pad, nk_pad;
-  int world, rank;
-  int causal, window, is_bf16;
-  float scale, softclamp;
-  PosMap pos;
-  int q_pos_offset;
-  int hop_count;
-  int hop_owner[kMaxWorld];  // K/V owners visited, hop 0 is this rank
+struct AttnBwdFusedParams : AttnProblem {
+  int n_pad, nk_pad;
   int self_owner[1];         // = {rank}: the streamed queries are always local
   const float* stat;
-  const uint32_t* kmask_bits;  // [world][batch][kmask_words]
-  int kmask_words;
   const uint32_t* ready;
   uint32_t ready_target;
   void* dk;

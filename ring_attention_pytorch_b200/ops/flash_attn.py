@@ -106,7 +106,7 @@ def _pad_d(t: Tensor, d_pad: int) -> Tensor:
 
 def _kernel_hop_forward(q, k, v, keep, causal, strict, scale, clamp):
     from ring_attention_pytorch_b200.ops import _ext
-    from ring_attention_pytorch_b200.ops.fused import alloc_kv_buffer, fused_attn_fwd, pack_key_mask_bits
+    from ring_attention_pytorch_b200.ops.fused import AttnProblem, alloc_kv_buffer, fused_attn_fwd, pack_key_mask_bits
 
     ops = _ext.ops()
     b, n_q, h, d = q.shape
@@ -119,9 +119,8 @@ def _kernel_hop_forward(q, k, v, keep, causal, strict, scale, clamp):
     kbits = pack_key_mask_bits(keep[None]) if keep is not None else None
     pm = make_position_map("plain", 1, n_k)
     # strict causal (diagonal masked) == causal with every query position shifted down by one
-    o, lse = fused_attn_fwd(qp, kv, [0], ready, kbits, kv_heads=hk, rank=0, pm=pm, causal=causal, window=None,
-                            scale=scale, softclamp=clamp, q_pos_offset=-1 if (causal and strict) else 0,
-                            hop_owner=[0])
+    prob = AttnProblem(b, h, hk, 0, pm, causal, None, scale, clamp, q_pos_offset=-1 if (causal and strict) else 0)
+    o, lse = fused_attn_fwd(prob, qp, kv, [0], ready, kbits)
     lse = torch.where(torch.isinf(lse), torch.full_like(lse, NEG_MAX), lse)
     return o[..., :d].float(), lse
 
@@ -229,8 +228,8 @@ def _dense_hop_backward(do, q, k, v, o, lse, bias, causal, strict, scale, clamp)
 
 def _kernel_hop_backward(do, q, k, v, o, lse, keep, causal, strict, scale, clamp):
     from ring_attention_pytorch_b200.ops import _ext
-    from ring_attention_pytorch_b200.ops.fused import (alloc_kv_buffer, alloc_qdo_buffer, alloc_stat_buffer,
-                                                       fused_attn_bwd, pack_key_mask_bits)
+    from ring_attention_pytorch_b200.ops.fused import (AttnProblem, alloc_kv_buffer, alloc_qdo_buffer,
+                                                       alloc_stat_buffer, fused_attn_bwd, pack_key_mask_bits)
 
     ops = _ext.ops()
     b, n_q, h, d = q.shape
@@ -246,9 +245,8 @@ def _kernel_hop_backward(do, q, k, v, o, lse, keep, causal, strict, scale, clamp
     ops.bwd_prep(qp, op, dop, lse_k, qdo, stat, 0)
     kbits = pack_key_mask_bits(keep[None]) if keep is not None else None
     pm = make_position_map("plain", 1, n_k)
-    dq, dk, dv = fused_attn_bwd(qdo, kv, stat, kbits, batch=b, heads=h, kv_heads=hk, rank=0, pm=pm, causal=causal,
-                                window=None, scale=scale, softclamp=clamp,
-                                q_pos_offset=-1 if (causal and strict) else 0)
+    prob = AttnProblem(b, h, hk, 0, pm, causal, None, scale, clamp, q_pos_offset=-1 if (causal and strict) else 0)
+    dq, dk, dv = fused_attn_bwd(prob, qdo, kv, stat, kbits)
     delta = stat[0, 1].view(b, h, -1)[..., :n_q]
     return dq[..., :d], dk[..., :d], dv[..., :d], delta
 

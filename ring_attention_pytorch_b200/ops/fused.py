@@ -8,7 +8,8 @@ multi-hop fetch/ready-flag protocol be tested on a single GPU.
 """
 from __future__ import annotations
 
-from typing import List, Optional, Sequence
+from dataclasses import dataclass
+from typing import Callable, List, Optional, Sequence
 
 import torch
 
@@ -34,66 +35,68 @@ def alloc_kv_buffer(world: int, batch: int, kv_heads: int, n_k: int, d: int, dty
     return torch.empty(world, 2, batch * kv_heads, n_k, d, dtype=dtype, device=device)
 
 
-def fused_attn_fwd(
-    q: torch.Tensor,
-    kv_buf: torch.Tensor,
-    peer_ptrs: Sequence[int],
-    ready: torch.Tensor,
-    kmask_bits: Optional[torch.Tensor],
-    *,
-    kv_heads: int,
-    rank: int,
-    pm: PositionMap,
-    causal: bool,
-    window: Optional[int],
-    scale: float,
-    softclamp: float = 0.0,
-    q_pos_offset: int = 0,
-    hop_owner: Optional[List[int]] = None,
-):
-    if hop_owner is None:
-        hop_owner = ring_hop_owners(pm, rank, causal, window)
-    return _ext.ops().attn_fwd(
-        q, kv_buf, list(peer_ptrs), ready, kmask_bits, kv_heads, rank, bool(causal), int(window or 0), float(scale),
-        float(softclamp), pm.stride, pm.seg_len, pm.base0, pm.base1, int(q_pos_offset), list(hop_owner))
+@dataclass(frozen=True)
+class AttnProblem:
+    """The attention problem one ring rank's kernel launches share: shapes, ring position, masking and scaling.
+
+    :meth:`tail` gives the arguments every ``torch.ops.rab.attn_*`` op ends with, in schema order."""
+    batch: int
+    heads: int
+    kv_heads: int
+    rank: int
+    pm: PositionMap
+    causal: bool
+    window: Optional[int]
+    scale: float
+    softclamp: float = 0.0
+    q_pos_offset: int = 0
+
+    def kv_owners(self) -> List[int]:
+        """K/V owners this rank visits, itself first."""
+        return ring_hop_owners(self.pm, self.rank, self.causal, self.window)
+
+    def q_owners(self) -> List[int]:
+        """Ranks whose queries see this rank's keys, itself first."""
+        return ring_query_owners(self.pm, self.rank, self.causal, self.window)
+
+    def tail(self, hop_owner: Sequence[int], kmask_bits: Optional[torch.Tensor] = None) -> tuple:
+        pm = self.pm
+        return (kmask_bits, self.batch, self.heads, self.kv_heads, self.rank, bool(self.causal), int(self.window or 0),
+                float(self.scale), float(self.softclamp), pm.stride, pm.seg_len, pm.base0, pm.base1,
+                int(self.q_pos_offset), list(hop_owner))
 
 
-def fused_attn_fwd_hop(
-    q: torch.Tensor,
-    kv_slot: torch.Tensor,
-    owner: int,
-    world: int,
-    carry_o: torch.Tensor,
-    carry_ml: torch.Tensor,
-    kmask_bits: Optional[torch.Tensor],
-    *,
-    carry_in: bool,
-    carry_out: bool,
-    kv_heads: int,
-    rank: int,
-    pm: PositionMap,
-    causal: bool,
-    window: Optional[int],
-    scale: float,
-    softclamp: float = 0.0,
-    q_pos_offset: int = 0,
-):
-    """ONE ring hop of the forward (``memory="ring"``): ``q`` against owner ``owner``'s K/V slot ``[2, b*hk, n_k, d]``.
-
-    The online-softmax state travels between the per-hop launches in ``carry_o`` (fp32 ``[b, n_q, h, d]``, the
-    un-normalised O) and ``carry_ml`` (fp32 ``[2, b*h, n_q]``: running maximum / sum); the launch with
-    ``carry_out=False`` returns the final (o, lse).  The reference carries (o, m, lse) between its per-hop Triton
-    launches the same way (ring_flash_attention_cuda.py:143-173)."""
-    return _ext.ops().attn_fwd_hop(
-        q, kv_slot[None], int(owner), int(world), carry_o, carry_ml, bool(carry_in), bool(carry_out), kmask_bits,
-        kv_heads, rank, bool(causal), int(window or 0), float(scale), float(softclamp), pm.stride, pm.seg_len, pm.base0,
-        pm.base1, int(q_pos_offset))
+def fused_attn_fwd(prob: AttnProblem, q: torch.Tensor, kv_buf: torch.Tensor, peer_ptrs: Sequence[int],
+                   ready: torch.Tensor, kmask_bits: Optional[torch.Tensor] = None):
+    """The whole ring in one launch: ``kv_buf`` ``[world, 2, b*hk, n_k, d]`` holds this rank's slot, the kernel's
+    fetchers pull owner o's slot from ``peer_ptrs[o]`` (0: already in ``kv_buf``).  Returns (o, lse)."""
+    return _ext.ops().attn_fwd(q, kv_buf, list(peer_ptrs), ready, *prob.tail(prob.kv_owners(), kmask_bits))
 
 
 def alloc_fwd_carry(q: torch.Tensor):
     b, n_q, h, d = q.shape
     return (torch.empty(b, n_q, h, d, dtype=torch.float32, device=q.device),
             torch.empty(2, b * h, n_q, dtype=torch.float32, device=q.device))
+
+
+def _no_hook(s: int) -> None:
+    pass
+
+
+def forward_hops(ops, prob: AttnProblem, q: torch.Tensor, hops: Sequence[int], slot: Callable[[int], torch.Tensor],
+                 kmask_bits: Optional[torch.Tensor] = None, launched: Callable[[int], None] = _no_hook):
+    """The forward one ring hop per launch (``memory="ring"``): hop ``s`` runs ``q`` against ``slot(s)``, owner
+    ``hops[s]``'s K/V ``[2, b*hk, n_k, d]``; ``launched(s)`` follows each launch.
+
+    The online-softmax state travels between the launches in fp32 carry buffers (un-normalised O, running maximum /
+    sum); the last launch returns the final (o, lse).  The reference carries (o, m, lse) between its per-hop Triton
+    launches the same way (ring_flash_attention_cuda.py:143-173)."""
+    carry_o, carry_ml = alloc_fwd_carry(q)
+    for s, owner in enumerate(hops):
+        o, lse = ops.attn_fwd_hop(q, slot(s)[None], carry_o, carry_ml, s > 0, s + 1 < len(hops),
+                                  *prob.tail([owner], kmask_bits))
+        launched(s)
+    return o, lse
 
 
 def emulate_ring_forward(
@@ -129,23 +132,16 @@ def emulate_ring_forward(
     if key_masks is not None:
         kbits = pack_key_mask_bits(torch.stack(list(key_masks), 0))
     outs, lses = [], []
-    if hopwise:
-        for r in range(world):
-            q = qs[r].contiguous()
-            carry_o, carry_ml = alloc_fwd_carry(q)
-            hops = ring_hop_owners(pm, r, causal, window)
-            for s_, owner in enumerate(hops):
-                o, lse = fused_attn_fwd_hop(q, bufs[owner][owner], owner, world, carry_o, carry_ml, kbits,
-                                            carry_in=s_ > 0, carry_out=s_ + 1 < len(hops), kv_heads=hk, rank=r, pm=pm,
-                                            causal=causal, window=window, scale=scale, softclamp=softclamp)
-            outs.append(o)
-            lses.append(lse)
-        return outs, lses
     for r in range(world):
-        ready = torch.zeros(world, dtype=torch.int32, device=dev)
-        peers = [bufs[o][o].data_ptr() for o in range(world)]  # owner o's own slot
-        o, lse = fused_attn_fwd(qs[r].contiguous(), bufs[r], peers, ready, kbits, kv_heads=hk, rank=r, pm=pm,
-                                causal=causal, window=window, scale=scale, softclamp=softclamp)
+        prob = AttnProblem(b, h, hk, r, pm, causal, window, scale, softclamp)
+        q = qs[r].contiguous()
+        if hopwise:
+            hops = prob.kv_owners()
+            o, lse = forward_hops(ops, prob, q, hops, lambda s: bufs[hops[s]][hops[s]], kbits)
+        else:
+            ready = torch.zeros(world, dtype=torch.int32, device=dev)
+            peers = [bufs[o][o].data_ptr() for o in range(world)]  # owner o's own slot
+            o, lse = fused_attn_fwd(prob, q, bufs[r], peers, ready, kbits)
         outs.append(o)
         lses.append(lse)
     return outs, lses
@@ -163,34 +159,12 @@ def alloc_stat_buffer(world: int, batch: int, heads: int, n_q: int, device) -> t
     return torch.zeros(world, 2, batch * heads, pad64(n_q), dtype=torch.float32, device=device)
 
 
-def fused_attn_bwd(
-    qdo_buf: torch.Tensor,
-    kv_buf: torch.Tensor,
-    stat_buf: torch.Tensor,
-    kmask_bits: Optional[torch.Tensor],
-    *,
-    batch: int,
-    heads: int,
-    kv_heads: int,
-    rank: int,
-    pm: PositionMap,
-    causal: bool,
-    window: Optional[int],
-    scale: float,
-    softclamp: float = 0.0,
-    q_pos_offset: int = 0,
-    ready_kv: Optional[torch.Tensor] = None,
-    ready_q: Optional[torch.Tensor] = None,
-    ready_target: int = 0,
-):
+def fused_attn_bwd(prob: AttnProblem, qdo_buf: torch.Tensor, kv_buf: torch.Tensor, stat_buf: torch.Tensor,
+                   kmask_bits: Optional[torch.Tensor] = None):
     """Run both backward kernels on already gathered buffers; returns (dq, dk, dv)."""
     ops = _ext.ops()
-    kv_owners = ring_hop_owners(pm, rank, causal, window)
-    q_owners = ring_query_owners(pm, rank, causal, window)
-    common = (kmask_bits, batch, heads, kv_heads, rank, bool(causal), int(window or 0), float(scale), float(softclamp),
-              pm.stride, pm.seg_len, pm.base0, pm.base1, int(q_pos_offset))
-    dq = ops.attn_bwd_dq(qdo_buf, kv_buf, stat_buf, ready_kv, ready_target, *common, kv_owners)
-    dk, dv = ops.attn_bwd_dkdv(qdo_buf, kv_buf, stat_buf, ready_q, ready_target, *common, q_owners)
+    dq = ops.attn_bwd_dq(qdo_buf, kv_buf, stat_buf, None, 0, *prob.tail(prob.kv_owners(), kmask_bits))
+    dk, dv = ops.attn_bwd_dkdv(qdo_buf, kv_buf, stat_buf, None, 0, *prob.tail(prob.q_owners(), kmask_bits))
     return dq, dk, dv
 
 
@@ -199,51 +173,44 @@ def pad128(n: int) -> int:
 
 
 def fused_attn_bwd_ring(
+    prob: AttnProblem,
     qdo: torch.Tensor,
     stat: torch.Tensor,
     kv_buf: torch.Tensor,
-    kmask_bits: Optional[torch.Tensor],
+    kmask_bits: Optional[torch.Tensor] = None,
     *,
-    batch: int,
-    heads: int,
-    kv_heads: int,
-    rank: int,
-    pm: PositionMap,
-    causal: bool,
-    window: Optional[int],
-    scale: float,
-    softclamp: float = 0.0,
-    q_pos_offset: int = 0,
     dq_acc: Optional[torch.Tensor] = None,
     dkv_acc_ptrs: Sequence[int] = (),
     nk_pad: int = 0,
     ready: Optional[torch.Tensor] = None,
     ready_target: int = 0,
-    hop_owner: Optional[List[int]] = None,
-    world: int = 0,
-    slot_owner: int = -1,
 ):
-    """The one-kernel (5-GEMM) backward, head dim 128 (``csrc/attn_bwd_fused_sm100.cu``).
+    """The one-kernel (5-GEMM) backward over every owner's K/V, head dim 128 (``csrc/attn_bwd_fused_sm100.cu``).
 
-    ``slot_owner >= 0`` (``memory="ring"``): ``kv_buf`` is ONE owner's slot ``[1, 2, b*hk, n_k, d]`` of a ``world``
-    rank ring and the launch covers that hop only; ``dq_acc`` and the dK/dV accumulators add up across the launches.
-
-    ``qdo`` [2, b*h, n_q, d] / ``stat`` [2, b*h, n_pad] are this rank's ``bwd_prep`` output, ``kv_buf`` the K/V gather.
+    ``qdo`` [2, b*h, n_q, d] / ``stat`` [2, b*h, n_pad] are this rank's ``bwd_prep`` output, ``kv_buf`` the K/V gather
+    (slot o usable once ``ready[o] >= ready_target``; no flags: all usable).
     dQ (unscaled) is added into ``dq_acc`` (fp32 [b*h, n_pad, d], allocated zeroed when not given).  Without
     ``dkv_acc_ptrs`` dK / dV come back as 16-bit tensors; with them (one fp32 [2, b*hk, nk_pad, d] accumulator address
     per ring rank) the kernel adds its tiles into the owners' accumulators and returns empty tensors.
     Returns (dq_acc, dk, dv)."""
-    ops = _ext.ops()
-    d = kv_buf.shape[-1]
     if dq_acc is None:
-        dq_acc = torch.zeros(batch * heads, stat.shape[-1], d, dtype=torch.float32, device=kv_buf.device)
-    if hop_owner is None:
-        hop_owner = ring_hop_owners(pm, rank, causal, window)
-    dk, dv = ops.attn_bwd_ring(qdo, kv_buf, stat, dq_acc, ready, int(ready_target), kmask_bits, batch, heads, kv_heads,
-                               rank, bool(causal), int(window or 0), float(scale), float(softclamp), pm.stride,
-                               pm.seg_len, pm.base0, pm.base1, int(q_pos_offset), list(hop_owner),
-                               list(dkv_acc_ptrs), int(nk_pad), int(world), int(slot_owner))
+        dq_acc = torch.zeros(prob.batch * prob.heads, stat.shape[-1], kv_buf.shape[-1], dtype=torch.float32,
+                             device=kv_buf.device)
+    dk, dv = _ext.ops().attn_bwd_ring(qdo, kv_buf, stat, dq_acc, ready, int(ready_target), list(dkv_acc_ptrs),
+                                      int(nk_pad), *prob.tail(prob.kv_owners(), kmask_bits))
     return dq_acc, dk, dv
+
+
+def backward_hops(ops, prob: AttnProblem, qdo: torch.Tensor, stat: torch.Tensor, dq_acc: torch.Tensor,
+                  hops: Sequence[int], slot: Callable[[int], torch.Tensor], *, dkv_acc_ptrs: Sequence[int],
+                  nk_pad: int, kmask_bits: Optional[torch.Tensor] = None, launched: Callable[[int], None] = _no_hook):
+    """The one-kernel backward one ring hop per launch (``memory="ring"``): hop ``s`` runs against ``slot(s)``, owner
+    ``hops[s]``'s K/V ``[2, b*hk, n_k, d]``; ``launched(s)`` follows each launch.  dQ adds up in ``dq_acc``, dK / dV
+    in the owners' accumulators ``dkv_acc_ptrs``, across the launches."""
+    for s, owner in enumerate(hops):
+        ops.attn_bwd_ring(qdo, slot(s)[None], stat, dq_acc, None, 0, list(dkv_acc_ptrs), int(nk_pad),
+                          *prob.tail([owner], kmask_bits))
+        launched(s)
 
 
 def emulate_ring_backward(
@@ -289,17 +256,16 @@ def emulate_ring_backward(
         ptrs = [a.data_ptr() for a in accs]
         dqs, direct = [], []
         for r in range(world):
+            prob = AttnProblem(b, h, hk, r, pm, causal, window, scale, softclamp)
             if hopwise and ring:
-                dq_acc = None
-                for owner in ring_hop_owners(pm, r, causal, window):
-                    dq_acc, dk, dv = fused_attn_bwd_ring(
-                        qdo_all[r], stat_all[r], kv_all[owner:owner + 1], kbits, batch=b, heads=h, kv_heads=hk, rank=r,
-                        pm=pm, causal=causal, window=window, scale=scale, softclamp=softclamp, dq_acc=dq_acc,
-                        dkv_acc_ptrs=ptrs, nk_pad=nk_pad, hop_owner=[owner], world=world, slot_owner=owner)
+                hops = prob.kv_owners()
+                dq_acc = torch.zeros(b * h, stat_all.shape[-1], d, dtype=torch.float32, device=dev)
+                backward_hops(ops, prob, qdo_all[r], stat_all[r], dq_acc, hops, lambda s: kv_all[hops[s]],
+                              dkv_acc_ptrs=ptrs, nk_pad=nk_pad, kmask_bits=kbits)
+                dk = dv = None
             else:
-                dq_acc, dk, dv = fused_attn_bwd_ring(qdo_all[r], stat_all[r], kv_all, kbits, batch=b, heads=h,
-                                                     kv_heads=hk, rank=r, pm=pm, causal=causal, window=window,
-                                                     scale=scale, softclamp=softclamp, dkv_acc_ptrs=ptrs, nk_pad=nk_pad)
+                dq_acc, dk, dv = fused_attn_bwd_ring(prob, qdo_all[r], stat_all[r], kv_all, kbits, dkv_acc_ptrs=ptrs,
+                                                     nk_pad=nk_pad)
             dqs.append(dq_acc)
             direct.append((dk, dv))
         for r in range(world):
@@ -316,6 +282,6 @@ def emulate_ring_backward(
         return res
     for r in range(world):
         # every emulated rank sees the same fully gathered buffers (what the NVLink gather produces)
-        res.append(fused_attn_bwd(qdo_all, kv_all, stat_all, kbits, batch=b, heads=h, kv_heads=hk, rank=r, pm=pm,
-                                  causal=causal, window=window, scale=scale, softclamp=softclamp))
+        res.append(fused_attn_bwd(AttnProblem(b, h, hk, r, pm, causal, window, scale, softclamp), qdo_all, kv_all,
+                                  stat_all, kbits))
     return res

@@ -49,18 +49,19 @@ from torch.autograd import Function
 
 from ring_attention_pytorch_b200.ops import _ext
 from ring_attention_pytorch_b200.ops.fused import (
-    alloc_fwd_carry,
+    AttnProblem,
     alloc_kv_buffer,
     alloc_qdo_buffer,
     alloc_stat_buffer,
+    backward_hops,
+    forward_hops,
     fused_attn_bwd_ring,
     fused_attn_fwd,
-    fused_attn_fwd_hop,
     pack_key_mask_bits,
     pad128,
 )
 from ring_attention_pytorch_b200.parallel.distributed import default, exists, get_rank, get_world_size, is_distributed
-from ring_attention_pytorch_b200.parallel.layout import make_position_map, ring_hop_owners, ring_query_owners
+from ring_attention_pytorch_b200.parallel.layout import make_position_map
 from ring_attention_pytorch_b200.parallel.symm import get_workspace
 from ring_attention_pytorch_b200.utils.timing import nvtx_range
 from ring_attention_pytorch_b200.utils.validate import check_attention_inputs, typecheck
@@ -110,10 +111,15 @@ def _gather_ring_masks(mask: Tensor, ring_size: int) -> Tensor:
     return torch.stack(gathered[ring_set * ring_size:(ring_set + 1) * ring_size]).bool()
 
 
+def _slot_bytes(b, hk, n_k, d_pad) -> int:
+    """Bytes of one owner's K/V slot ``[2, b*hk, n_k, d]`` (16 bit)."""
+    return 2 * b * hk * n_k * d_pad * 2
+
+
 def _ring_gather_workspace(ws, ring_size, b, hk, n_k, d_pad, dt):
     """This call's K/V gather buffer ``[W, 2, b*hk, n_k, d]`` inside the symmetric workspace (double buffered across
     calls) and, per ring rank, the address of THAT rank's own slot in ITS buffer (what the fetchers pull from)."""
-    slot_bytes = 2 * b * hk * n_k * d_pad * 2
+    slot_bytes = _slot_bytes(b, hk, n_k, d_pad)
     local, bases = ws.staging("kv_gather", ring_size * slot_bytes)
     gather = local[:ring_size * slot_bytes].view(dt).view(ring_size, 2, b * hk, n_k, d_pad)
     own_slot_ptrs = [bases[o] + o * slot_bytes for o in range(ring_size)]
@@ -123,9 +129,27 @@ def _ring_gather_workspace(ws, ring_size, b, hk, n_k, d_pad, dt):
 def _own_slot_workspace(ws, b, hk, n_k, d_pad, dt):
     """``memory="ring"``: this rank's own K/V slot ``[2, b*hk, n_k, d]`` in symmetric memory (double buffered across
     calls) and every ring rank's address of ITS slot."""
-    slot_bytes = 2 * b * hk * n_k * d_pad * 2
+    slot_bytes = _slot_bytes(b, hk, n_k, d_pad)
     local, bases = ws.staging("kv_own", slot_bytes)
     return local[:slot_bytes].view(dt).view(2, b * hk, n_k, d_pad), bases, slot_bytes
+
+
+def _place_kv(ws, hop_mode: bool, rank: int, ring_size: int, b, hk, n_k, d_pad, dt, dev):
+    """Where this rank packs its K/V and what the kernels read it through: ``(target, kv_buf, own_ptrs, slot_bytes)``.
+
+    ``target`` is the ``[2, b*hk, n_k, d]`` slot to pack into; ``own_ptrs[o]`` is ring rank o's address of ITS own
+    slot, what the peers pull from.
+      hop mode (``memory="ring"``): this rank's own symmetric slot; ``kv_buf`` is None (the kernels read a _HopWindow)
+      gather: slot ``rank`` of the W-slot symmetric gather buffer ``kv_buf``
+      single rank (``ws`` is None): slot 0 of a local 1-slot ``kv_buf``; no ``own_ptrs``"""
+    if ws is None:
+        kv = alloc_kv_buffer(1, b, hk, n_k, d_pad, dt, dev)
+        return kv[0], kv, None, _slot_bytes(b, hk, n_k, d_pad)
+    if hop_mode:
+        own, own_ptrs, slot_bytes = _own_slot_workspace(ws, b, hk, n_k, d_pad, dt)
+        return own, None, own_ptrs, slot_bytes
+    gather, own_ptrs, slot_bytes = _ring_gather_workspace(ws, ring_size, b, hk, n_k, d_pad, dt)
+    return gather[rank], gather, own_ptrs, slot_bytes
 
 
 class _HopWindow:
@@ -248,60 +272,39 @@ class RingFlashAttentionCUDAFunction(Function):
         rank = get_rank() % ring_size if use_ring else 0
         pm = make_position_map(layout, ring_size, n_k)
         q_off = (n_k - n_q) if (cross_attn and causal) else 0
+        softclamp = float(softclamp_value) if softclamp_qk_sim else 0.0
+        prob = AttnProblem(b, h, hk, rank, pm, causal, max_lookback_seq_len, scale, softclamp, q_off)
         dev = q.device
 
-        ready = torch.zeros(ring_size, dtype=torch.int32, device=dev)
-        peers = [0] * ring_size
-        kbits = None
-        hop_mode = use_ring and _use_hop_window(2 * b * hk * n_k * d_pad * 2)
+        hop_mode = use_ring and _use_hop_window(_slot_bytes(b, hk, n_k, d_pad))
+        ws = get_workspace(ring_size, dev) if use_ring else None
         with nvtx_range("rab.fwd.pack+barrier"):
-            if hop_mode:
-                ws = get_workspace(ring_size, dev)
-                own, own_ptrs, slot_bytes = _own_slot_workspace(ws, b, hk, n_k, d_pad, dt)
-                _pack_slot(ops, kp, vp, own, ang if fused_k_rotary else None)
+            own, kv_gather, own_ptrs, slot_bytes = _place_kv(ws, hop_mode, rank, ring_size, b, hk, n_k, d_pad, dt, dev)
+            _pack_slot(ops, kp, vp, own, ang if fused_k_rotary else None)
+            _count()
+            kbits = None
+            if use_ring:
                 ws.barrier()  # every peer's own slot is complete
-                _count(2)
-                kv_gather = None
-                if exists(mask):
-                    kbits = pack_key_mask_bits(_gather_ring_masks(mask, ring_size))
-            elif use_ring:
-                ws = get_workspace(ring_size, dev)
-                kv_gather, own_slot_ptrs, _ = _ring_gather_workspace(ws, ring_size, b, hk, n_k, d_pad, dt)
-                _pack_slot(ops, kp, vp, kv_gather[rank], ang if fused_k_rotary else None)
-                ws.barrier()  # every peer's own slot is complete
-                _count(2)
-                peers = [0 if o == rank else own_slot_ptrs[o] for o in range(ring_size)]
-                if exists(mask):
-                    kbits = pack_key_mask_bits(_gather_ring_masks(mask, ring_size))
-            else:
-                kv_gather = alloc_kv_buffer(1, b, hk, n_k, d_pad, dt, dev)
-                _pack_slot(ops, kp, vp, kv_gather[0], ang if fused_k_rotary else None)
                 _count()
                 if exists(mask):
-                    kbits = pack_key_mask_bits(mask[None])
+                    kbits = pack_key_mask_bits(_gather_ring_masks(mask, ring_size))
+            elif exists(mask):
+                kbits = pack_key_mask_bits(mask[None])
 
-        softclamp = float(softclamp_value) if softclamp_qk_sim else 0.0
         with nvtx_range("rab.fwd.kernel"):
             if hop_mode:
-                hops = ring_hop_owners(pm, rank, causal, max_lookback_seq_len)
+                hops = prob.kv_owners()
                 window_slots = _HopWindow(ops, ws, own, own_ptrs, slot_bytes, hops)
-                carry_o, carry_ml = alloc_fwd_carry(qp)
-                for s_, owner in enumerate(hops):
-                    o, lse = fused_attn_fwd_hop(qp, window_slots.slot(s_), owner, ring_size, carry_o, carry_ml, kbits,
-                                                carry_in=s_ > 0, carry_out=s_ + 1 < len(hops), kv_heads=hk, rank=rank,
-                                                pm=pm, causal=causal, window=max_lookback_seq_len, scale=scale,
-                                                softclamp=softclamp, q_pos_offset=q_off)
-                    window_slots.launched(s_)
-                    _count()
-                del carry_o, carry_ml
+                o, lse = forward_hops(ops, prob, qp, hops, window_slots.slot, kbits, window_slots.launched)
+                _count(len(hops))
             else:
-                o, lse = fused_attn_fwd(qp, kv_gather, peers, ready, kbits, kv_heads=hk, rank=rank, pm=pm,
-                                        causal=causal, window=max_lookback_seq_len, scale=scale, softclamp=softclamp,
-                                        q_pos_offset=q_off)
+                ready = torch.zeros(ring_size, dtype=torch.int32, device=dev)
+                peers = [0 if o_ == rank else own_ptrs[o_] for o_ in range(ring_size)] if use_ring else [0]
+                o, lse = fused_attn_fwd(prob, qp, kv_gather, peers, ready, kbits)
                 _count()
 
-        ctx.cfg = (causal, max_lookback_seq_len, ring_size, rank, layout, softclamp, scale, q_off, use_ring, d, d_pad,
-                   orig_dtype, hk, fused_k_rotary)
+        ctx.prob = prob
+        ctx.cfg = (ring_size, rank, use_ring, d, d_pad, orig_dtype, fused_k_rotary)
         # single rank: the packed K/V is exactly what the backward needs; ring: keep the (small) inputs, re-pack later
         none = torch.empty(0, device=dev)
         ctx.save_for_backward(qp, kp if use_ring else none, vp if use_ring else none, o, lse,
@@ -313,33 +316,26 @@ class RingFlashAttentionCUDAFunction(Function):
     @staticmethod
     def backward(ctx, do: Tensor):
         ops = _ext.ops()
-        (causal, window, ring_size, rank, layout, softclamp, scale, q_off, use_ring, d, d_pad, orig_dtype,
-         hk, fused_k_rotary) = ctx.cfg
+        prob = ctx.prob
+        ring_size, rank, use_ring, d, d_pad, orig_dtype, fused_k_rotary = ctx.cfg
         qp, kp, vp, o, lse, kv_saved, kbits, ang = ctx.saved_tensors
         kbits = kbits if kbits.numel() > 0 else None
         ang = ang if ang.numel() > 0 else None
         dt = qp.dtype
         b, n_q, h, _ = qp.shape
+        hk = prob.kv_heads
         dev = qp.device
         dop = _pad_head_dim(do.to(dt), d_pad).contiguous()
         n_k = kp.shape[1] if use_ring else kv_saved.shape[3]
-        pm = make_position_map(layout, ring_size, n_k)
-        hop_owner = ring_hop_owners(pm, rank, causal, window)
+        hop_owner = prob.kv_owners()
 
-        ws = None
-        kv_own_ptrs, kv_bytes = None, 0
+        ws, kv_own_ptrs, kv_bytes = None, None, 0
         hop_mode = (use_ring and d_pad == 128 and CONFIG["backward"] == "fused"
-                    and _use_hop_window(2 * b * hk * n_k * d_pad * 2))
-        if hop_mode:
+                    and _use_hop_window(_slot_bytes(b, hk, n_k, d_pad)))
+        if use_ring:  # re-pack this rank's own slot (the forward's buffers are long reused)
             ws = get_workspace(ring_size, dev)
-            own, kv_own_ptrs, kv_bytes = _own_slot_workspace(ws, b, hk, n_k, d_pad, dt)
+            own, kv_gather, kv_own_ptrs, kv_bytes = _place_kv(ws, hop_mode, rank, ring_size, b, hk, n_k, d_pad, dt, dev)
             _pack_slot(ops, kp, vp, own, ang if fused_k_rotary else None)
-            _count()
-            kv_gather = None
-        elif use_ring:  # rebuild the gather buffer around this rank's own slot (the forward's buffer is long reused)
-            ws = get_workspace(ring_size, dev)
-            kv_gather, kv_own_ptrs, kv_bytes = _ring_gather_workspace(ws, ring_size, b, hk, n_k, d_pad, dt)
-            _pack_slot(ops, kp, vp, kv_gather[rank], ang if fused_k_rotary else None)
             _count()
         else:
             kv_gather = kv_saved
@@ -386,24 +382,18 @@ class RingFlashAttentionCUDAFunction(Function):
             with nvtx_range("rab.bwd.kernel"):
                 if hop_mode:  # one launch per hop against the 2-slot window; dq_acc / the owners' dK, dV accumulate
                     window_slots = _HopWindow(ops, ws, own, kv_own_ptrs, kv_bytes, hop_owner)
-                    for s_, owner in enumerate(hop_owner):
-                        fused_attn_bwd_ring(qdo[0], stat[0], window_slots.slot(s_)[None], kbits, batch=b, heads=h,
-                                            kv_heads=hk, rank=rank, pm=pm, causal=causal, window=window, scale=scale,
-                                            softclamp=softclamp, q_pos_offset=q_off, dq_acc=dq_acc,
-                                            dkv_acc_ptrs=acc_ptrs, nk_pad=nk_pad, hop_owner=[owner], world=ring_size,
-                                            slot_owner=owner)
-                        window_slots.launched(s_)
-                        _count()
-                    _count(-1)
+                    backward_hops(ops, prob, qdo[0], stat[0], dq_acc, hop_owner, window_slots.slot,
+                                  dkv_acc_ptrs=acc_ptrs, nk_pad=nk_pad, kmask_bits=kbits,
+                                  launched=window_slots.launched)
+                    _count(len(hop_owner))
                 else:
-                    _, dk, dv = fused_attn_bwd_ring(qdo[0], stat[0], kv_gather, kbits, batch=b, heads=h, kv_heads=hk,
-                                                    rank=rank, pm=pm, causal=causal, window=window, scale=scale,
-                                                    softclamp=softclamp, q_pos_offset=q_off, dq_acc=dq_acc,
+                    _, dk, dv = fused_attn_bwd_ring(prob, qdo[0], stat[0], kv_gather, kbits, dq_acc=dq_acc,
                                                     dkv_acc_ptrs=acc_ptrs, nk_pad=nk_pad, ready=ready,
-                                                    ready_target=ready_target, hop_owner=hop_owner)
+                                                    ready_target=ready_target)
+                    _count()
                 dq = torch.empty(b, n_q, h, d_pad, dtype=dt, device=dev)
-                ops.acc_convert(dq_acc, dq, scale)
-                _count(2)
+                ops.acc_convert(dq_acc, dq, prob.scale)
+                _count()
             if use_ring:
                 with nvtx_range("rab.bwd.barrier+convert"):
                     if side_done is not None:
@@ -430,24 +420,20 @@ class RingFlashAttentionCUDAFunction(Function):
                 ws.barrier()
                 _count(3)
                 ready_kv, _ = pull_kv_slots()  # K/V first: the dQ kernel consumes it hop by hop
-                q_owners = ring_query_owners(pm, rank, causal, window)
                 with torch.cuda.stream(ws.side_stream):
-                    for o_rank in q_owners[1:]:
+                    for o_rank in prob.q_owners()[1:]:
                         ops.peer_copy(qdo_gather[o_rank], peer_ptrs[o_rank], qdo_bytes)
                         ops.peer_copy(stat_gather[o_rank], peer_ptrs[o_rank] + qdo_bytes, stat_bytes)
                     gather_done = torch.cuda.Event()
                     gather_done.record(ws.side_stream)
                 qdo_gather.record_stream(ws.side_stream)
                 stat_gather.record_stream(ws.side_stream)
-            common = (kbits, b, h, hk, rank, bool(causal), int(window or 0), float(scale), float(softclamp), pm.stride,
-                      pm.seg_len, pm.base0, pm.base1, int(q_off))
             # dQ only needs the K/V slots (flag per owner): it overlaps with the Q/dO gather
-            dq = ops.attn_bwd_dq(qdo_gather, kv_gather, stat_gather, ready_kv, 1 if ready_kv is not None else 0, *common,
-                                 hop_owner)
+            dq = ops.attn_bwd_dq(qdo_gather, kv_gather, stat_gather, ready_kv, 1 if ready_kv is not None else 0,
+                                 *prob.tail(hop_owner, kbits))
             if gather_done is not None:
                 torch.cuda.current_stream(dev).wait_event(gather_done)
-            dk, dv = ops.attn_bwd_dkdv(qdo_gather, kv_gather, stat_gather, None, 0, *common,
-                                       ring_query_owners(pm, rank, causal, window))
+            dk, dv = ops.attn_bwd_dkdv(qdo_gather, kv_gather, stat_gather, None, 0, *prob.tail(prob.q_owners(), kbits))
             _count(2)
 
         dq, dk, dv = dq[..., :d], dk[..., :d], dv[..., :d]

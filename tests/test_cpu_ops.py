@@ -189,7 +189,7 @@ def test_blockwise_feedforward_matches_plain_and_shares_state_dict():
 
 def test_poly_exp2_reference():
     """Host emulation (fp32 op by op) of ``poly_exp2x2`` in csrc/ptx.cuh, the FMA-pipe exponential the forward kernel
-    can use for a share of its softmax (RAB_FWD_EXP_POLY): relative error < 1.5e-4, masked logits give exactly 0."""
+    runs for a quarter of its softmax (POLYQ in csrc/attn_fwd_sm100.cu): relative error < 1.5e-4, masked logits give exactly 0."""
     import numpy as np
 
     c = np.array([1.0, 0.6932103037834167, 0.24221116304397583, 0.05536489188671112], dtype=np.float32)

@@ -43,7 +43,7 @@ def main():
     dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
 
     from ring_attention_pytorch_b200.ops import _ext
-    from ring_attention_pytorch_b200.ops.fused import fused_attn_fwd
+    from ring_attention_pytorch_b200.ops.fused import AttnProblem, fused_attn_fwd
     from ring_attention_pytorch_b200.ops.ring_cuda import _ring_gather_workspace
     from ring_attention_pytorch_b200.parallel.layout import make_position_map
     from ring_attention_pytorch_b200.parallel.symm import get_workspace
@@ -55,6 +55,7 @@ def main():
     dt = torch.bfloat16
     ws = get_workspace(world, dev)
     pm = make_position_map("plain", world, n_k)
+    prob = AttnProblem(b, 1, hk, rank, pm, False, None, d ** -0.5)
     q = torch.randn(b, 128, 1, d, device=dev, dtype=dt)
     k = torch.randn(b, n_k, hk, d, device=dev, dtype=dt)
     v = torch.randn(b, n_k, hk, d, device=dev, dtype=dt)
@@ -72,8 +73,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         # non-causal: every owner is visited, 128 queries x n_k keys of one head per owner: microseconds of MMA work
-        fused_attn_fwd(q, gather, peers, ready, None, kv_heads=hk, rank=rank, pm=pm, causal=False, window=None,
-                       scale=d ** -0.5)
+        fused_attn_fwd(prob, q, gather, peers, ready)
         e1.record()
         torch.cuda.synchronize()
         ops.set_fetch_timing(None)

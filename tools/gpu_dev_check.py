@@ -190,8 +190,8 @@ def case_perf_bwd_fused(n=16384, h=16, causal=True, iters=5, b=1, hk=None):
     """The one-kernel backward (prep + kernel + dQ convert), timed like case_perf_bwd."""
     import torch
     from ring_attention_pytorch_b200.ops import _ext
-    from ring_attention_pytorch_b200.ops.fused import (alloc_kv_buffer, alloc_qdo_buffer, alloc_stat_buffer,
-                                                       fused_attn_bwd_ring, fused_attn_fwd)
+    from ring_attention_pytorch_b200.ops.fused import (AttnProblem, alloc_kv_buffer, alloc_qdo_buffer,
+                                                       alloc_stat_buffer, fused_attn_bwd_ring, fused_attn_fwd)
     from ring_attention_pytorch_b200.parallel.layout import make_position_map
 
     ops = _ext.ops()
@@ -208,8 +208,8 @@ def case_perf_bwd_fused(n=16384, h=16, causal=True, iters=5, b=1, hk=None):
     stat = alloc_stat_buffer(1, b, h, n, "cuda")
     ops.pack_kv(k, v, kv[0])
     ready = torch.zeros(1, dtype=torch.int32, device="cuda")
-    o, lse = fused_attn_fwd(q, kv, [0], ready, None, kv_heads=hk, rank=0, pm=pm, causal=causal, window=None,
-                            scale=d ** -0.5)
+    prob = AttnProblem(b, h, hk, 0, pm, causal, None, d ** -0.5)
+    o, lse = fused_attn_fwd(prob, q, kv, [0], ready)
     dq = torch.empty_like(q)
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
 
@@ -222,8 +222,7 @@ def case_perf_bwd_fused(n=16384, h=16, causal=True, iters=5, b=1, hk=None):
         acc = torch.zeros(b * h, stat.shape[-1], d, dtype=torch.float32, device="cuda")
         if timed:
             ev[2].record()
-        _, dk, dv = fused_attn_bwd_ring(qdo[0], stat[0], kv, None, batch=b, heads=h, kv_heads=hk, rank=0, pm=pm,
-                                        causal=causal, window=None, scale=d ** -0.5, dq_acc=acc)
+        _, dk, dv = fused_attn_bwd_ring(prob, qdo[0], stat[0], kv, dq_acc=acc)
         if timed:
             ev[3].record()
         ops.acc_convert(acc, dq, d ** -0.5)
@@ -255,8 +254,8 @@ def case_perf_bwd_fused(n=16384, h=16, causal=True, iters=5, b=1, hk=None):
 def case_perf_bwd(n=16384, h=16, d=128, causal=True, iters=5, b=1, hk=None):
     import torch
     from ring_attention_pytorch_b200.ops import _ext
-    from ring_attention_pytorch_b200.ops.fused import (alloc_kv_buffer, alloc_qdo_buffer, alloc_stat_buffer,
-                                                       fused_attn_bwd, fused_attn_fwd)
+    from ring_attention_pytorch_b200.ops.fused import (AttnProblem, alloc_kv_buffer, alloc_qdo_buffer,
+                                                       alloc_stat_buffer, fused_attn_bwd, fused_attn_fwd)
     from ring_attention_pytorch_b200.parallel.layout import make_position_map
 
     ops = _ext.ops()
@@ -272,13 +271,12 @@ def case_perf_bwd(n=16384, h=16, d=128, causal=True, iters=5, b=1, hk=None):
     stat = alloc_stat_buffer(1, b, h, n, "cuda")
     ops.pack_kv(k, v, kv[0])
     ready = torch.zeros(1, dtype=torch.int32, device="cuda")
-    o, lse = fused_attn_fwd(q, kv, [0], ready, None, kv_heads=hk, rank=0, pm=pm, causal=causal, window=None,
-                            scale=d ** -0.5)
+    prob = AttnProblem(b, h, hk, 0, pm, causal, None, d ** -0.5)
+    o, lse = fused_attn_fwd(prob, q, kv, [0], ready)
 
     def run():
         ops.bwd_prep(q, o, do, lse, qdo, stat, 0)
-        return fused_attn_bwd(qdo, kv, stat, None, batch=b, heads=h, kv_heads=hk, rank=0, pm=pm, causal=causal,
-                              window=None, scale=d ** -0.5)
+        return fused_attn_bwd(prob, qdo, kv, stat)
 
     for _ in range(2):
         run()
@@ -296,13 +294,12 @@ def case_perf_bwd(n=16384, h=16, d=128, causal=True, iters=5, b=1, hk=None):
     res = {"ms": ms, "tflops_5gemm_equiv": flops / ms / 1e9, "tflops_executed_7gemm": flops * 1.4 / ms / 1e9}
     # per-kernel split
     e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
-    common = (None, b, h, hk, 0, causal, 0, d ** -0.5, 0.0, pm.stride, pm.seg_len, pm.base0, pm.base1, 0)
     e[0].record()
     ops.bwd_prep(q, o, do, lse, qdo, stat, 0)
     e[1].record()
-    ops.attn_bwd_dq(qdo, kv, stat, None, 0, *common, [0])
+    ops.attn_bwd_dq(qdo, kv, stat, None, 0, *prob.tail([0]))
     e[2].record()
-    ops.attn_bwd_dkdv(qdo, kv, stat, None, 0, *common, [0])
+    ops.attn_bwd_dkdv(qdo, kv, stat, None, 0, *prob.tail([0]))
     e[3].record()
     torch.cuda.synchronize()
     res["ms_prep"], res["ms_dq"], res["ms_dkdv"] = e[0].elapsed_time(e[1]), e[1].elapsed_time(e[2]), e[2].elapsed_time(e[3])
@@ -367,10 +364,10 @@ def case_perf_hop(world=4, n=16384, h=8, hk=None, d=128, layout="striped", causa
     same K/V slots (already local: no transfer in either arm), forward and one-kernel backward."""
     import torch
     from ring_attention_pytorch_b200.ops import _ext
-    from ring_attention_pytorch_b200.ops.fused import (alloc_fwd_carry, alloc_kv_buffer, alloc_qdo_buffer,
-                                                       alloc_stat_buffer, fused_attn_bwd_ring, fused_attn_fwd,
-                                                       fused_attn_fwd_hop, pad128)
-    from ring_attention_pytorch_b200.parallel.layout import make_position_map, ring_hop_owners
+    from ring_attention_pytorch_b200.ops.fused import (AttnProblem, alloc_kv_buffer, alloc_qdo_buffer,
+                                                       alloc_stat_buffer, backward_hops, forward_hops,
+                                                       fused_attn_bwd_ring, fused_attn_fwd, pad128)
+    from ring_attention_pytorch_b200.parallel.layout import make_position_map
 
     ops = _ext.ops()
     hk = hk or h
@@ -383,23 +380,19 @@ def case_perf_hop(world=4, n=16384, h=8, hk=None, d=128, layout="striped", causa
         ops.pack_kv(torch.randn(b, n, hk, d, device="cuda", dtype=dt), torch.randn(b, n, hk, d, device="cuda", dtype=dt),
                     buf[o_])
     pm = make_position_map(layout, world, n)
-    hops = ring_hop_owners(pm, rank, causal, None)
+    prob = AttnProblem(b, h, hk, rank, pm, causal, None, d ** -0.5)
+    hops = prob.kv_owners()
     ready = torch.zeros(world, dtype=torch.int32, device="cuda")
-    peers = [0] * world  # every slot is local: the fetchers copy slot -> slot (same bytes a real ring pulls)
-    kw = dict(kv_heads=hk, rank=rank, pm=pm, causal=causal, window=None, scale=d ** -0.5)
-    carry_o, carry_ml = alloc_fwd_carry(q)
     accs = [torch.zeros(2, b * hk, pad128(n), d, dtype=torch.float32, device="cuda") for _ in range(world)]
     ptrs = [a.data_ptr() for a in accs]
     state = {}
 
     def fwd_single():
-        state["o"], state["lse"] = fused_attn_fwd(q, buf, [buf[o_].data_ptr() if o_ != rank else 0 for o_ in range(world)],
-                                                  ready, None, **kw)
+        state["o"], state["lse"] = fused_attn_fwd(prob, q, buf, [buf[o_].data_ptr() if o_ != rank else 0
+                                                                 for o_ in range(world)], ready)
 
     def fwd_hop():
-        for s_, owner in enumerate(hops):
-            state["o"], state["lse"] = fused_attn_fwd_hop(q, buf[owner], owner, world, carry_o, carry_ml, None,
-                                                          carry_in=s_ > 0, carry_out=s_ + 1 < len(hops), **kw)
+        state["o"], state["lse"] = forward_hops(ops, prob, q, hops, lambda s: buf[hops[s]])
 
     def prep():
         qdo = alloc_qdo_buffer(1, b, h, n, d, dt, "cuda")
@@ -408,14 +401,12 @@ def case_perf_hop(world=4, n=16384, h=8, hk=None, d=128, layout="striped", causa
         return qdo, stat
 
     def bwd_single():
-        fused_attn_bwd_ring(state["qdo"][0], state["stat"][0], buf, None, batch=b, heads=h, dq_acc=state["dq"],
-                            dkv_acc_ptrs=ptrs, nk_pad=pad128(n), **kw)
+        fused_attn_bwd_ring(prob, state["qdo"][0], state["stat"][0], buf, dq_acc=state["dq"], dkv_acc_ptrs=ptrs,
+                            nk_pad=pad128(n))
 
     def bwd_hop():
-        for owner in hops:
-            fused_attn_bwd_ring(state["qdo"][0], state["stat"][0], buf[owner:owner + 1], None, batch=b, heads=h,
-                                dq_acc=state["dq"], dkv_acc_ptrs=ptrs, nk_pad=pad128(n), hop_owner=[owner], world=world,
-                                slot_owner=owner, **kw)
+        backward_hops(ops, prob, state["qdo"][0], state["stat"][0], state["dq"], hops, lambda s: buf[hops[s]],
+                      dkv_acc_ptrs=ptrs, nk_pad=pad128(n))
 
     def timeit(fn):
         for _ in range(2):
@@ -452,7 +443,7 @@ def case_perf_hop(world=4, n=16384, h=8, hk=None, d=128, layout="striped", causa
 def case_perf(n=16384, h=16, d=128, causal=True, iters=5, b=1, hk=None):
     import torch
     from ring_attention_pytorch_b200.ops import _ext
-    from ring_attention_pytorch_b200.ops.fused import alloc_kv_buffer, fused_attn_fwd
+    from ring_attention_pytorch_b200.ops.fused import AttnProblem, alloc_kv_buffer, fused_attn_fwd
     from ring_attention_pytorch_b200.parallel.layout import make_position_map
 
     ops = _ext.ops()
@@ -466,9 +457,10 @@ def case_perf(n=16384, h=16, d=128, causal=True, iters=5, b=1, hk=None):
     ops.pack_kv(k, v, buf[0])
     ready = torch.zeros(1, dtype=torch.int32, device="cuda")
 
+    prob = AttnProblem(b, h, hk, 0, pm, causal, None, d ** -0.5)
+
     def run():
-        return fused_attn_fwd(q, buf, [0], ready, None, kv_heads=hk, rank=0, pm=pm, causal=causal, window=None,
-                              scale=d ** -0.5)
+        return fused_attn_fwd(prob, q, buf, [0], ready)
 
     for _ in range(2):
         run()

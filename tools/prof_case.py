@@ -13,8 +13,9 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ring_attention_pytorch_b200.ops import _ext  # noqa: E402
-from ring_attention_pytorch_b200.ops.fused import (alloc_kv_buffer, alloc_qdo_buffer, alloc_stat_buffer,  # noqa: E402
-                                                   fused_attn_bwd, fused_attn_bwd_ring, fused_attn_fwd)
+from ring_attention_pytorch_b200.ops.fused import (AttnProblem, alloc_kv_buffer, alloc_qdo_buffer,  # noqa: E402
+                                                   alloc_stat_buffer, fused_attn_bwd, fused_attn_bwd_ring,
+                                                   fused_attn_fwd)
 from ring_attention_pytorch_b200.ops.tree_decode_cuda import tree_decode_cuda  # noqa: E402
 from ring_attention_pytorch_b200.parallel.layout import make_position_map  # noqa: E402
 
@@ -26,20 +27,19 @@ ops = _ext.ops()
 dt = torch.bfloat16
 q, k, v, do = (torch.randn(1, n, h, d, device="cuda", dtype=dt) for _ in range(4))
 pm = make_position_map("plain", 1, n)
+prob = AttnProblem(1, h, h, 0, pm, causal, None, d ** -0.5)
 kv = alloc_kv_buffer(1, 1, h, n, d, dt, "cuda")
 qdo = alloc_qdo_buffer(1, 1, h, n, d, dt, "cuda")
 stat = alloc_stat_buffer(1, 1, h, n, "cuda")
 ready = torch.zeros(1, dtype=torch.int32, device="cuda")
 ops.pack_kv(k, v, kv[0])
-o, lse = fused_attn_fwd(q, kv, [0], ready, None, kv_heads=h, rank=0, pm=pm, causal=causal, window=None, scale=d ** -0.5)
+o, lse = fused_attn_fwd(prob, q, kv, [0], ready)
 ops.bwd_prep(q, o, do, lse, qdo, stat, 0)
 if d == 128:
-    dq_acc, dk, dv = fused_attn_bwd_ring(qdo[0], stat[0], kv, None, batch=1, heads=h, kv_heads=h, rank=0, pm=pm, causal=causal,
-                                         window=None, scale=d ** -0.5)
+    dq_acc, dk, dv = fused_attn_bwd_ring(prob, qdo[0], stat[0], kv)
     dq = torch.empty_like(q)
     ops.acc_convert(dq_acc, dq, d ** -0.5)
-fused_attn_bwd(qdo, kv, stat, None, batch=1, heads=h, kv_heads=h, rank=0, pm=pm, causal=causal, window=None,
-               scale=d ** -0.5)
+fused_attn_bwd(prob, qdo, kv, stat)
 # decode: 8192 keys, batch 64, 32 / 8 heads
 qd = torch.randn(64, 32, 1, 128, device="cuda", dtype=dt)
 kd = torch.randn(64, 8, 8192, 128, device="cuda", dtype=dt)
