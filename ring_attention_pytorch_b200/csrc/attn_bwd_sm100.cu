@@ -19,7 +19,10 @@
 // This pair is the backward of head dim 64 and the deterministic alternative at head dim 128, where the default is
 // the one-kernel, 5-GEMM backward in attn_bwd_fused_sm100.cu.
 //
-// Inputs are the *gathered* ring buffers (see kernels.h); remote slots are published through ready flags.
+// Inputs are the *gathered* ring buffers (see kernels.h); remote slots are published through ready flags.  In hop mode
+// (memory = "ring", one launch per ring hop) the softmax warpgroups load each item's accumulator rows from the fp32
+// carry into TMEM before the first accumulating MMA and the epilogue stores them back: the launches perform the same
+// fp32 operations in the same order as one launch over every hop.
 #include "attn_common.cuh"
 
 namespace rab {
@@ -54,8 +57,62 @@ struct DqSmem {
   uint64_t v_full[2], v_empty[2];
   uint64_t r_s_full[3], r_s_taken[3], r_dp_full[3], r_ds_ready[3], r_free[3];  // per TMEM region
   uint64_t dq_done, epi_done;
+  uint64_t carry_ready;  // hop mode: both warpgroups have loaded the item's carried dQ into TMEM
   uint32_t tmem_base;
 };
+
+// Before an item's first accumulating MMA the accumulating issuer waits until the accumulator block is its own: the
+// previous item's epilogue has drained it, or (hop mode) the warpgroups have loaded the carried accumulator into it,
+// which they do only after that epilogue.  Either barrier completes once per item, and the warpgroups arrive for item
+// i + 1 only after the issuer's commit of item i, which follows this wait: neither can run two phases ahead.
+__device__ __forceinline__ void wait_acc_free(const AttnBwdParams& p, uint64_t* epi_done, uint64_t* carry_ready,
+                                              uint32_t n_item, int tag) {
+  if (p.carry_in) mbar_wait(carry_ready, n_item & 1, tag + 1);
+  else mbar_wait(epi_done, (n_item & 1) ^ 1, tag);
+}
+
+// hop mode: one thread's row of its warpgroup's accumulator columns, fp32 carry -> TMEM (zeros for rows past the end)
+template <int NCOL>
+__device__ __forceinline__ void carry_load(const float* src, bool row_ok, uint32_t taddr) {
+  const float4* crow = reinterpret_cast<const float4*>(src);
+#pragma unroll 1
+  for (int c = 0; c < NCOL; c += 32) {
+    uint32_t v[32];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const float4 x = row_ok ? crow[c / 4 + i] : make_float4(0.f, 0.f, 0.f, 0.f);
+      v[4 * i + 0] = __float_as_uint(x.x);
+      v[4 * i + 1] = __float_as_uint(x.y);
+      v[4 * i + 2] = __float_as_uint(x.z);
+      v[4 * i + 3] = __float_as_uint(x.w);
+    }
+    tmem_st32(taddr + c, v);
+  }
+  tc_wait_st();
+}
+
+// hop mode: TMEM -> fp32 carry (zeros when the accumulator was never written)
+template <int NCOL>
+__device__ __forceinline__ void carry_store(float* dst, bool row_ok, bool any, uint32_t taddr) {
+  float4* crow = reinterpret_cast<float4*>(dst);
+#pragma unroll 1
+  for (int c = 0; c < NCOL; c += 32) {
+    uint32_t v[32];
+    if (any) {
+      tmem_ld32(taddr + c, v);
+      tc_wait_ld();
+    } else {
+#pragma unroll
+      for (int i = 0; i < 32; ++i) v[i] = 0u;
+    }
+    if (row_ok) {
+#pragma unroll
+      for (int i = 0; i < 8; ++i)
+        crow[c / 4 + i] = make_float4(__uint_as_float(v[4 * i]), __uint_as_float(v[4 * i + 1]),
+                                      __uint_as_float(v[4 * i + 2]), __uint_as_float(v[4 * i + 3]));
+    }
+  }
+}
 
 struct DqItem {
   int b, h, kvh, qt, row0;
@@ -242,11 +299,11 @@ __device__ __forceinline__ void dq_issue_dq(DqSmem<D>& sm, const AttnBwdParams& 
       const uint32_t g = tile_base + j;
       const uint32_t r = g % 3, ph = (g / 3) & 1;
       mbar_wait(&sm.r_ds_ready[r], ph, 660 + r);
-      if (j == 0) mbar_wait(&sm.epi_done, (n_item & 1) ^ 1, 610);
+      if (j == 0) wait_acc_free(p, &sm.epi_done, &sm.carry_ready, n_item, 610);
       tc_fence_after();
       const uint32_t x_tm = tmem + dq_region_col(r);
       const uint64_t kmn = k_mndesc0 + uint64_t(r * SLOT16);
-      const uint32_t acc0 = j > 0 ? 1u : 0u;
+      const uint32_t acc0 = (j > 0 || p.carry_in) ? 1u : 0u;
       if (elect_one()) {
 #pragma unroll
         for (int kk = 0; kk < 128 / 16; ++kk) {
@@ -257,7 +314,7 @@ __device__ __forceinline__ void dq_issue_dq(DqSmem<D>& sm, const AttnBwdParams& 
       }
       __syncwarp();
     }
-    if (ntiles == 0) mbar_wait(&sm.epi_done, (n_item & 1) ^ 1, 611);
+    if (ntiles == 0) wait_acc_free(p, &sm.epi_done, &sm.carry_ready, n_item, 612);
     umma_commit_w(&sm.dq_done);
     tile_base += ntiles;
   }
@@ -288,6 +345,14 @@ __device__ __forceinline__ void dq_softmax(DqSmem<D>& sm, const AttnBwdParams& p
     if (row_ok) {
       lse2 = p.stat[stat_row + grow];
       delta = p.stat[stat_row + (size_t)p.batch * p.heads * p.n_pad + grow];
+    }
+    // hop mode: columns [W*D/2, (W+1)*D/2) of this row's dQ continue from the previous hop's launch (this thread
+    // drained them in the previous item's epilogue)
+    auto dq_row = [&]() { return (((size_t)it.b * p.n_q + (row_ok ? grow : 0)) * p.heads + it.h) * D + W * (D / 2); };
+    if (p.carry_in) {
+      carry_load<D / 2>(p.carry + dq_row(), row_ok, dq_tm + W * (D / 2));
+      tc_fence_before();
+      mbar_arrive(&sm.carry_ready);
     }
 
     DqScan scan;
@@ -424,11 +489,13 @@ __device__ __forceinline__ void dq_softmax(DqSmem<D>& sm, const AttnBwdParams& p
     // epilogue: warpgroup W converts columns [W*D/2, (W+1)*D/2) of dQ
     mbar_wait(&sm.dq_done, n_item & 1, 720 + W);
     tc_fence_after();
-    {
-      // the item may have had no visible tile at all: dQ is then zero and TMEM holds stale data
-      const bool any = jj > 0;
-      uint16_t* drow = reinterpret_cast<uint16_t*>(p.dq) +
-                       (((size_t)it.b * p.n_q + (row_ok ? grow : 0)) * p.heads + it.h) * D + W * (D / 2);
+    if (p.carry_out) {
+      // an item with no visible tile leaves a carried accumulator as it is
+      if (jj > 0 || !p.carry_in) carry_store<D / 2>(p.carry + dq_row(), row_ok, jj > 0, dq_tm + W * (D / 2));
+    } else {
+      // the item may have had no visible tile at all: dQ is then zero (or the carry) and TMEM holds stale data
+      const bool any = jj > 0 || p.carry_in;
+      uint16_t* drow = reinterpret_cast<uint16_t*>(p.dq) + dq_row();
 #pragma unroll
       for (int c = 0; c < D / 2; c += 32) {
         uint32_t acc[32];
@@ -484,6 +551,7 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap map_qd, const __grid_cons
     }
     mbar_init(&sm.dq_done, 1);
     mbar_init(&sm.epi_done, 256);
+    mbar_init(&sm.carry_ready, 256);
     fence_mbar_init();
   }
   if (warp == 10) {
@@ -528,6 +596,7 @@ struct DkvSmem {
   uint64_t qd_full[QSTAGES], qd_empty[QSTAGES];
   uint64_t s_full[2], s_free[2], dp_full[2], pds_ready[2];
   uint64_t acc_done, epi_done;
+  uint64_t carry_ready;  // hop mode: both warpgroups have loaded the item's carried dK / dV into TMEM
   uint32_t tmem_base;
 };
 
@@ -726,11 +795,11 @@ __device__ __forceinline__ void dkv_issue_acc(DkvSmem<D>& sm, const AttnBwdParam
       const uint32_t w = j & 1u;
       const uint32_t st = (tile_base + j) % QSTAGES;
       mbar_wait(&sm.pds_ready[w], c_b[w] & 1, 940 + w);
-      if (j == 0) mbar_wait(&sm.epi_done, (n_item & 1) ^ 1, 910);
+      if (j == 0) wait_acc_free(p, &sm.epi_done, &sm.carry_ready, n_item, 910);
       tc_fence_after();
       const uint32_t y_tm = tmem + w * 128u + 64u;
       const uint64_t qmn = q_mndesc0 + uint64_t(st * STAGE16), domn = do_mndesc0 + uint64_t(st * STAGE16);
-      const uint32_t acc0 = j > 0 ? 1u : 0u;
+      const uint32_t acc0 = (j > 0 || p.carry_in) ? 1u : 0u;
       if (elect_one()) {
 #pragma unroll
         for (int kk = 0; kk < 64 / 16; ++kk) {
@@ -746,7 +815,7 @@ __device__ __forceinline__ void dkv_issue_acc(DkvSmem<D>& sm, const AttnBwdParam
       c_b[w]++;
       if (j + 2 < ntiles) issue_dp(j + 2);
     }
-    if (ntiles == 0) mbar_wait(&sm.epi_done, (n_item & 1) ^ 1, 911);
+    if (ntiles == 0) wait_acc_free(p, &sm.epi_done, &sm.carry_ready, n_item, 912);
     umma_commit_w(&sm.acc_done);
     umma_commit_w(&sm.kv_empty);
     tile_base += ntiles;
@@ -777,6 +846,17 @@ __device__ __forceinline__ void dkv_softmax(DkvSmem<D>& sm, const AttnBwdParams&
     if (key_ok && p.kmask_bits != nullptr) {
       const uint32_t wbits = p.kmask_bits[((size_t)p.rank * p.batch + it.b) * p.kmask_words + (key >> 5)];
       key_ok = (wbits >> (key & 31)) & 1u;
+    }
+    // warpgroup 0 owns dK, warpgroup 1 dV: in hop mode this key's row continues from the previous hop's launch (this
+    // thread drained it in the previous item's epilogue)
+    auto carry_row = [&]() {
+      return p.carry + (size_t)W * p.batch * p.n_k * p.kv_heads * D +
+             (((size_t)it.b * p.n_k + (key < p.n_k ? key : 0)) * p.kv_heads + it.kvh) * D;
+    };
+    if (p.carry_in) {
+      carry_load<D>(carry_row(), key < p.n_k, tmem + 256 + (W == 0 ? 0 : D) + lane_off);
+      tc_fence_before();
+      mbar_arrive(&sm.carry_ready);
     }
 
     DkvScan scan;
@@ -899,10 +979,13 @@ __device__ __forceinline__ void dkv_softmax(DkvSmem<D>& sm, const AttnBwdParams&
     // epilogue: warpgroup 0 writes dK, warpgroup 1 writes dV
     mbar_wait(&sm.acc_done, n_item & 1, 1010 + W);
     tc_fence_after();
-    {
-      const bool any = jn > 0;
-      const uint32_t acc_tm = tmem + 256 + (W == 0 ? 0 : D) + lane_off;
-      const bool row_ok = key < p.n_k;
+    const bool row_ok = key < p.n_k;
+    const uint32_t acc_tm = tmem + 256 + (W == 0 ? 0 : D) + lane_off;
+    if (p.carry_out) {
+      // an item with no visible tile leaves a carried accumulator as it is
+      if (jn > 0 || !p.carry_in) carry_store<D>(carry_row(), row_ok, jn > 0, acc_tm);
+    } else {
+      const bool any = jn > 0 || p.carry_in;
       uint16_t* out = reinterpret_cast<uint16_t*>(W == 0 ? p.dk : p.dv) +
                       (((size_t)it.b * p.n_k + (row_ok ? key : 0)) * p.kv_heads + it.kvh) * D;
 #pragma unroll
@@ -956,6 +1039,7 @@ attn_bwd_dkdv_kernel(const __grid_constant__ CUtensorMap map_qd64, const __grid_
     }
     mbar_init(&sm.acc_done, 1);
     mbar_init(&sm.epi_done, 256);
+    mbar_init(&sm.carry_ready, 256);
     fence_mbar_init();
   }
   if (warp == 10) {

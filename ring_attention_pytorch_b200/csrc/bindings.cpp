@@ -165,21 +165,23 @@ void parse_problem(rab::AttnProblem& p, const Tensor& kv_buf, int n_q, PROBLEM_P
   }
 }
 
-// Address of owner slot 0 as the kernels see it.  They address owner o's K / V at slot o; a one-slot buffer IS slot
-// hop_owner[0], so its base moves down by that many slots (only that slot is ever dereferenced).
-uint8_t* kv_slot0(const Tensor& kv_buf, const rab::AttnProblem& p) {
-  const size_t slot_bytes = kv_buf.nbytes() / kv_buf.size(0);
-  const int shift = kv_buf.size(0) == p.world ? 0 : p.hop_owner[0];
-  return reinterpret_cast<uint8_t*>(kv_buf.data_ptr()) - shift * slot_bytes;
+// Address of owner slot 0 of a per-owner buffer [slots][...] as the kernels see it.  They address owner o's data at
+// slot o: a buffer with every owner's slot is used as it is, and a one-slot buffer IS the slot of `owner`, so its base
+// moves down by that many slots (only that slot is ever dereferenced).
+uint8_t* slot0(const Tensor& buf, int world, int owner) {
+  const size_t slot_bytes = buf.nbytes() / buf.size(0);
+  const int shift = buf.size(0) == world ? 0 : owner;
+  return reinterpret_cast<uint8_t*>(buf.data_ptr()) - shift * slot_bytes;
 }
 
-// K/V of every owner, [world][2][b*hk][n_k][d] -> dims (d, n_k, b*hk, 2*world), box (64, 128, 1, 1)
-CUtensorMap make_kv_map(const Tensor& kv_buf, const rab::AttnProblem& p) {
+// K/V of every owner, [world][2][b*hk][n_k][d] -> dims (d, n_k, b*hk, 2*world), box (64, 128, 1, 1); a one-slot
+// kv_buf is the slot of `owner`
+CUtensorMap make_kv_map(const Tensor& kv_buf, const rab::AttnProblem& p, int owner) {
   const uint64_t d = kv_buf.size(4), rows = (uint64_t)p.batch * p.kv_heads;
   uint64_t dims[4] = {d, (uint64_t)p.n_k, rows, (uint64_t)2 * p.world};
   uint64_t str[3] = {d * 2, (uint64_t)p.n_k * d * 2, rows * p.n_k * d * 2};
   uint32_t box[4] = {64, 128, 1, 1};
-  return rab::make_tmap_bf16(kv_slot0(kv_buf, p), 4, dims, str, box, rab::TmapSwizzle::B128);
+  return rab::make_tmap_bf16(slot0(kv_buf, p.world, owner), 4, dims, str, box, rab::TmapSwizzle::B128);
 }
 
 // per-owner ready flags: int32, one per ring rank (null when not given)
@@ -201,7 +203,7 @@ void parse_fwd(rab::AttnFwdParams& p, const Tensor& q, const Tensor& kv_buf, PRO
   TORCH_CHECK(kv_buf.scalar_type() == q.scalar_type());
   TORCH_CHECK(q.size(0) == batch && q.size(2) == heads && q.size(3) == kv_buf.size(4));
   p.slot_bytes = kv_buf.nbytes() / kv_buf.size(0);
-  p.kv_local = kv_slot0(kv_buf, p);
+  p.kv_local = slot0(kv_buf, p.world, p.hop_owner[0]);
 }
 
 std::tuple<Tensor, Tensor> launch_fwd(const Tensor& q, const Tensor& kv_buf, rab::AttnFwdParams& p) {
@@ -216,7 +218,7 @@ std::tuple<Tensor, Tensor> launch_fwd(const Tensor& q, const Tensor& kv_buf, rab
   uint64_t qstr[3] = {(uint64_t)d * 2, (uint64_t)h * d * 2, (uint64_t)n_q * h * d * 2};
   uint32_t qbox[4] = {64, 1, 128, 1};
   CUtensorMap map_q = rab::make_tmap_bf16(q.data_ptr(), 4, qdims, qstr, qbox, rab::TmapSwizzle::B128);
-  CUtensorMap map_kv = make_kv_map(kv_buf, p);
+  CUtensorMap map_kv = make_kv_map(kv_buf, p, p.hop_owner[0]);
   auto stream = at::cuda::getCurrentCUDAStream();
   if (d == 128) {
     rab::launch_attn_fwd<128>(map_q, map_kv, p, sm_count(), stream);
@@ -290,10 +292,11 @@ struct BwdSetup {
   CUtensorMap map_qd128, map_qd64, map_kv;
 };
 
-// the two-kernel backward: qdo_buf [world][2][b*h][n_q][d], kv_buf [world][2][b*hk][n_k][d], stat_buf
-// [world][2][b*h][n_pad], all gathered
-BwdSetup make_bwd_setup(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
-                        const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
+// The two-kernel backward's buffers: qdo_buf [slots][2][b*h][n_q][d], kv_buf [slots][2][b*hk][n_k][d], stat_buf
+// [slots][2][b*h][n_pad].  Each holds every owner's slot (gathered, slots = world) or the one slot of qdo_owner /
+// kv_owner (the Q/dO buffer and the statistics share their owner).
+BwdSetup make_bwd_setup(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf, bool one_slot,
+                        bool kv_is_own, PROBLEM_PARAMS) {
   check_16bit(qdo_buf, "qdo_buf");
   TORCH_CHECK(qdo_buf.is_contiguous() && stat_buf.is_contiguous());
   TORCH_CHECK(qdo_buf.dim() == 5 && stat_buf.dim() == 4);
@@ -302,30 +305,61 @@ BwdSetup make_bwd_setup(const Tensor& qdo_buf, const Tensor& kv_buf, const Tenso
   std::memset(&p, 0, sizeof(p));
   parse_problem(p, kv_buf, (int)qdo_buf.size(3), PROBLEM_ARGS);
   const int world = p.world, n_q = p.n_q, d = kv_buf.size(4);
-  TORCH_CHECK(kv_buf.size(0) == world, "the two-kernel backward needs every owner's slot");
-  TORCH_CHECK(qdo_buf.size(0) == world && qdo_buf.size(2) == batch * heads && qdo_buf.size(4) == d);
-  TORCH_CHECK(stat_buf.size(0) == world && stat_buf.size(2) == batch * heads);
+  const int slots = one_slot ? 1 : world;
+  TORCH_CHECK(kv_buf.size(0) == slots, one_slot ? "one owner's K/V slot expected" :
+              "the two-kernel backward needs every owner's slot");
+  TORCH_CHECK(qdo_buf.scalar_type() == kv_buf.scalar_type(), "qdo_buf and kv_buf must share a dtype");
+  TORCH_CHECK(qdo_buf.size(0) == slots && qdo_buf.size(1) == 2 && qdo_buf.size(2) == batch * heads &&
+              qdo_buf.size(4) == d, "qdo_buf must be [slots, 2, b*h, n_q, d]");
+  TORCH_CHECK(stat_buf.size(0) == slots && stat_buf.size(1) == 2 && stat_buf.size(2) == batch * heads,
+              "stat_buf must be [slots, 2, b*h, n_pad]");
+  if (one_slot) {
+    TORCH_CHECK(stat_buf.scalar_type() == at::kFloat && stat_buf.size(3) % 64 == 0 && stat_buf.size(3) >= n_q,
+                "stat_buf must be fp32 with n_pad >= n_q, n_pad % 64 == 0");
+  }
+  // the dQ kernel reads this rank's queries against the hop owner's keys, the dK/dV kernel this rank's keys against
+  // the hop owner's queries
+  const int kv_owner = kv_is_own ? p.rank : p.hop_owner[0];
+  const int q_owner = kv_is_own ? p.hop_owner[0] : p.rank;
   p.n_pad = stat_buf.size(3);
-  p.stat = stat_buf.data_ptr<float>();
-  p.ready = ready_flags(ready, world);
-  p.ready_target = p.ready ? (uint32_t)ready_target : 0;
+  p.stat = reinterpret_cast<const float*>(slot0(stat_buf, world, q_owner));
   uint64_t qdims[4] = {(uint64_t)d, (uint64_t)n_q, (uint64_t)batch * heads, (uint64_t)2 * world};
   uint64_t qstr[3] = {(uint64_t)d * 2, (uint64_t)n_q * d * 2, (uint64_t)batch * heads * n_q * d * 2};
   uint32_t qbox128[4] = {64, 128, 1, 1};
   uint32_t qbox64[4] = {64, 64, 1, 1};
-  s.map_qd128 = rab::make_tmap_bf16(qdo_buf.data_ptr(), 4, qdims, qstr, qbox128, rab::TmapSwizzle::B128);
-  s.map_qd64 = rab::make_tmap_bf16(qdo_buf.data_ptr(), 4, qdims, qstr, qbox64, rab::TmapSwizzle::B128);
-  s.map_kv = make_kv_map(kv_buf, p);
+  uint8_t* qd0 = slot0(qdo_buf, world, q_owner);
+  s.map_qd128 = rab::make_tmap_bf16(qd0, 4, qdims, qstr, qbox128, rab::TmapSwizzle::B128);
+  s.map_qd64 = rab::make_tmap_bf16(qd0, 4, qdims, qstr, qbox64, rab::TmapSwizzle::B128);
+  s.map_kv = make_kv_map(kv_buf, p, kv_owner);
   return s;
 }
 
-Tensor attn_bwd_dq(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
-                   const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
-  c10::cuda::CUDAGuard guard(kv_buf.device());
-  BwdSetup s = make_bwd_setup(qdo_buf, kv_buf, stat_buf, ready, ready_target, PROBLEM_ARGS);
+// gathered buffers: slot o usable once ready[o] >= ready_target (no flags: all usable)
+BwdSetup make_bwd_gather_setup(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
+                               const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
+  BwdSetup s = make_bwd_setup(qdo_buf, kv_buf, stat_buf, false, false, PROBLEM_ARGS);
+  s.p.ready = ready_flags(ready, s.p.world);
+  s.p.ready_target = s.p.ready ? (uint32_t)ready_target : 0;
+  return s;
+}
+
+// one ring hop: `carry` holds the fp32 accumulators between the launches (see AttnBwdParams); unused, and then
+// unchecked, when neither flag is set
+void set_bwd_carry(rab::AttnBwdParams& p, Tensor& carry, at::IntArrayRef shape, bool carry_in, bool carry_out,
+                   const char* what) {
+  if (!carry_in && !carry_out) return;
+  TORCH_CHECK(carry.is_cuda() && carry.scalar_type() == at::kFloat && carry.is_contiguous() && carry.sizes() == shape,
+              "carry must be contiguous fp32 ", what, " ", shape);
+  p.carry = carry.data_ptr<float>();
+  p.carry_in = carry_in;
+  p.carry_out = carry_out;
+}
+
+// dQ [b, n_q, h, d] 16 bit, or (carry_out) an empty tensor: the accumulator stays in the carry
+Tensor launch_bwd_dq(BwdSetup& s, const Tensor& kv_buf, int64_t batch, int64_t heads) {
   const int d = kv_buf.size(4);
-  Tensor dq = torch::empty({batch, s.p.n_q, heads, d}, kv_buf.options());
-  s.p.dq = dq.data_ptr();
+  Tensor dq = torch::empty({s.p.carry_out ? 0 : batch, s.p.n_q, heads, d}, kv_buf.options());
+  s.p.dq = s.p.carry_out ? nullptr : dq.data_ptr();
   auto stream = at::cuda::getCurrentCUDAStream();
   if (d == 128) {
     rab::launch_attn_bwd_dq<128>(s.map_qd128, s.map_kv, s.p, sm_count(), stream);
@@ -335,15 +369,13 @@ Tensor attn_bwd_dq(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& st
   return dq;
 }
 
-std::tuple<Tensor, Tensor> attn_bwd_dkdv(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
-                                         const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
-  c10::cuda::CUDAGuard guard(kv_buf.device());
-  BwdSetup s = make_bwd_setup(qdo_buf, kv_buf, stat_buf, ready, ready_target, PROBLEM_ARGS);
+// dK, dV [b, n_k, hk, d] 16 bit, or (carry_out) empty tensors: the accumulators stay in the carry
+std::tuple<Tensor, Tensor> launch_bwd_dkdv(BwdSetup& s, const Tensor& kv_buf, int64_t batch, int64_t kv_heads) {
   const int d = kv_buf.size(4);
-  Tensor dk = torch::empty({batch, s.p.n_k, kv_heads, d}, kv_buf.options());
-  Tensor dv = torch::empty({batch, s.p.n_k, kv_heads, d}, kv_buf.options());
-  s.p.dk = dk.data_ptr();
-  s.p.dv = dv.data_ptr();
+  Tensor dk = torch::empty({s.p.carry_out ? 0 : batch, s.p.n_k, kv_heads, d}, kv_buf.options());
+  Tensor dv = torch::empty({s.p.carry_out ? 0 : batch, s.p.n_k, kv_heads, d}, kv_buf.options());
+  s.p.dk = s.p.carry_out ? nullptr : dk.data_ptr();
+  s.p.dv = s.p.carry_out ? nullptr : dv.data_ptr();
   auto stream = at::cuda::getCurrentCUDAStream();
   if (d == 128) {
     rab::launch_attn_bwd_dkdv<128>(s.map_qd64, s.map_kv, s.p, sm_count(), stream);
@@ -351,6 +383,43 @@ std::tuple<Tensor, Tensor> attn_bwd_dkdv(const Tensor& qdo_buf, const Tensor& kv
     rab::launch_attn_bwd_dkdv<64>(s.map_qd64, s.map_kv, s.p, sm_count(), stream);
   }
   return {dk, dv};
+}
+
+Tensor attn_bwd_dq(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
+                   const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
+  c10::cuda::CUDAGuard guard(kv_buf.device());
+  BwdSetup s = make_bwd_gather_setup(qdo_buf, kv_buf, stat_buf, ready, ready_target, PROBLEM_ARGS);
+  return launch_bwd_dq(s, kv_buf, batch, heads);
+}
+
+// One ring hop of the dQ kernel: this rank's qdo_own [1, 2, b*h, n_q, d] / stat_own [1, 2, b*h, n_pad] against the
+// one K/V slot kv_slot [1, 2, b*hk, n_k, d] of owner hop_owner[0].  carry fp32 [b, n_q, h, d] (unscaled dQ) travels
+// between the launches; with carry_out the result stays in it and an empty tensor is returned.
+Tensor attn_bwd_dq_hop(const Tensor& qdo_own, const Tensor& kv_slot, const Tensor& stat_own, Tensor carry,
+                       bool carry_in, bool carry_out, PROBLEM_PARAMS) {
+  c10::cuda::CUDAGuard guard(kv_slot.device());
+  BwdSetup s = make_bwd_setup(qdo_own, kv_slot, stat_own, true, false, PROBLEM_ARGS);
+  set_bwd_carry(s.p, carry, {batch, s.p.n_q, heads, kv_slot.size(4)}, carry_in, carry_out, "[b, n_q, h, d]");
+  return launch_bwd_dq(s, kv_slot, batch, heads);
+}
+
+std::tuple<Tensor, Tensor> attn_bwd_dkdv(const Tensor& qdo_buf, const Tensor& kv_buf, const Tensor& stat_buf,
+                                         const c10::optional<Tensor>& ready, int64_t ready_target, PROBLEM_PARAMS) {
+  c10::cuda::CUDAGuard guard(kv_buf.device());
+  BwdSetup s = make_bwd_gather_setup(qdo_buf, kv_buf, stat_buf, ready, ready_target, PROBLEM_ARGS);
+  return launch_bwd_dkdv(s, kv_buf, batch, kv_heads);
+}
+
+// One ring hop of the dK/dV kernel: this rank's kv_own [1, 2, b*hk, n_k, d] against the one Q/dO slot qdo_slot
+// [1, 2, b*h, n_q, d] / stat_slot [1, 2, b*h, n_pad] of query owner hop_owner[0].  carry fp32 [2, b, n_k, hk, d]
+// (unscaled dK, dV) travels between the launches; with carry_out the result stays in it and empty tensors are returned.
+std::tuple<Tensor, Tensor> attn_bwd_dkdv_hop(const Tensor& qdo_slot, const Tensor& kv_own, const Tensor& stat_slot,
+                                             Tensor carry, bool carry_in, bool carry_out, PROBLEM_PARAMS) {
+  c10::cuda::CUDAGuard guard(kv_own.device());
+  BwdSetup s = make_bwd_setup(qdo_slot, kv_own, stat_slot, true, true, PROBLEM_ARGS);
+  set_bwd_carry(s.p, carry, {2, batch, s.p.n_k, kv_heads, kv_own.size(4)}, carry_in, carry_out,
+                "[2, b, n_k, hk, d]");
+  return launch_bwd_dkdv(s, kv_own, batch, kv_heads);
 }
 
 // One-kernel (5-GEMM) ring backward, head dim 128 (attn_bwd_fused_sm100.cu).
@@ -391,7 +460,7 @@ std::tuple<Tensor, Tensor> attn_bwd_ring(const Tensor& qdo, const Tensor& kv_buf
   uint64_t qstr[3] = {(uint64_t)d * 2, (uint64_t)n_q * d * 2, (uint64_t)batch * heads * n_q * d * 2};
   uint32_t qbox64[4] = {64, 64, 1, 1};
   CUtensorMap map_qd64 = rab::make_tmap_bf16(qdo.data_ptr(), 4, qdims, qstr, qbox64, rab::TmapSwizzle::B128);
-  CUtensorMap map_kv = make_kv_map(kv_buf, p);
+  CUtensorMap map_kv = make_kv_map(kv_buf, p, p.hop_owner[0]);
   // dQ accumulator: 2-D (d, b*h*n_pad) fp32, box 32 columns x 32 rows, no swizzle (rows written lane-contiguous)
   uint64_t adims[2] = {(uint64_t)d, (uint64_t)batch * heads * n_pad};
   uint64_t astr[1] = {(uint64_t)d * 4};
@@ -653,6 +722,10 @@ TORCH_LIBRARY(rab, m) {
         ") -> Tensor");
   m.def("attn_bwd_dkdv(Tensor qdo_buf, Tensor kv_buf, Tensor stat_buf, Tensor? ready, int ready_target, " PROBLEM_SCHEMA
         ") -> (Tensor, Tensor)");
+  m.def("attn_bwd_dq_hop(Tensor qdo_own, Tensor kv_slot, Tensor stat_own, Tensor(a!) carry, bool carry_in, bool "
+        "carry_out, " PROBLEM_SCHEMA ") -> Tensor");
+  m.def("attn_bwd_dkdv_hop(Tensor qdo_slot, Tensor kv_own, Tensor stat_slot, Tensor(a!) carry, bool carry_in, bool "
+        "carry_out, " PROBLEM_SCHEMA ") -> (Tensor, Tensor)");
   m.def("attn_bwd_ring(Tensor qdo, Tensor kv_buf, Tensor stat, Tensor(a!) dq_acc, Tensor? ready, int ready_target, int[] "
         "dkv_acc_ptrs, int nk_pad, " PROBLEM_SCHEMA ") -> (Tensor, Tensor)");
   m.def("acc_convert(Tensor acc, Tensor(a!) out, float scale) -> ()");
@@ -675,6 +748,8 @@ TORCH_LIBRARY_IMPL(rab, CUDA, m) {
   m.impl("bwd_prep", &bwd_prep);
   m.impl("attn_bwd_dq", &attn_bwd_dq);
   m.impl("attn_bwd_dkdv", &attn_bwd_dkdv);
+  m.impl("attn_bwd_dq_hop", &attn_bwd_dq_hop);
+  m.impl("attn_bwd_dkdv_hop", &attn_bwd_dkdv_hop);
   m.impl("attn_bwd_ring", &attn_bwd_ring);
   m.impl("acc_convert", &acc_convert);
 }

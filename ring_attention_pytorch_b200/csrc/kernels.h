@@ -95,19 +95,25 @@ size_t attn_fwd_smem_bytes(int head_dim);
 // fused ring flash-attention backward: two kernels, no atomics, no cross-rank reduction.
 //   dq kernel   : Q-stationary  (like forward), streams K/V tiles of every visible owner
 //   dkdv kernel : KV-stationary, streams Q / dO / lse / delta tiles of every rank that can see the keys
-// Both read *gathered* buffers: kv_buf [world][2][b*hk][n_k][d] and qdo_buf [world][2][b*h][n_q][d]
-// (16 bit) plus stat_buf [world][2][b*h][n_pad] (fp32: lse*log2e, delta).  Slot `rank` is written
+// Both address kv_buf [world][2][b*hk][n_k][d] and qdo_buf [world][2][b*h][n_q][d] (16 bit) plus stat_buf
+// [world][2][b*h][n_pad] (fp32: lse*log2e, delta) by owner slot.  Gather mode: slot `rank` is written
 // locally, the other slots arrive over NVLink (copy engines on a side stream, or an earlier kernel) and
-// are published through the per-owner ready flags.
+// are published through the per-owner ready flags.  Hop mode (memory = "ring"): one launch per ring hop,
+// every buffer is one owner's slot (its base shifted so that the owner's slot index lands on it), and the
+// fp32 accumulators travel between the launches in `carry`.
 // ------------------------------------------------------------------------------------------------
 struct AttnBwdParams : AttnProblem {
   int n_pad;
-  const float* stat;           // gathered [world][2][b*h][n_pad]
+  const float* stat;           // [world][2][b*h][n_pad]
   void* dq;                    // [b, n_q, h, d]
   void* dk;                    // [b, n_k, hk, d]
   void* dv;                    // [b, n_k, hk, d]
   const uint32_t* ready;       // [world] flags: slot o usable once ready[o] >= ready_target (may be null)
   uint32_t ready_target;
+  // hop-at-a-time mode: dq kernel fp32 [b, n_q, h, d]; dkdv kernel fp32 [2][b, n_k, hk, d] (dK, dV); both unscaled
+  float* carry;
+  int carry_in;   // 1: every item's accumulator starts from `carry` instead of zero
+  int carry_out;  // 1: store the fp32 accumulator to `carry` instead of the scaled 16-bit output
 };
 
 template <int D>

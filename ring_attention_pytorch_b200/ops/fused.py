@@ -9,7 +9,7 @@ multi-hop fetch/ready-flag protocol be tested on a single GPU.
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import Callable, List, Optional, Sequence
+from typing import Callable, List, Optional, Sequence, Tuple
 
 import torch
 
@@ -213,6 +213,42 @@ def backward_hops(ops, prob: AttnProblem, qdo: torch.Tensor, stat: torch.Tensor,
         launched(s)
 
 
+def two_kernel_backward_hops(ops, prob: AttnProblem, qdo_own: torch.Tensor, stat_own: torch.Tensor,
+                             kv_slot: Callable[[int], torch.Tensor],
+                             qdo_slot: Callable[[int], Tuple[torch.Tensor, torch.Tensor]],
+                             kmask_bits: Optional[torch.Tensor] = None, launched: Callable[[int], None] = _no_hook):
+    """The two-kernel backward one ring hop per launch (``memory="ring"``).  Returns (dq, dk, dv).
+
+    Step ``s`` launches dQ hop ``s``: this rank's ``qdo_own`` [2, b*h, n_q, d] / ``stat_own`` [2, b*h, n_pad] against
+    ``kv_slot(s)``, the K/V [2, b*hk, n_k, d] of ``prob.kv_owners()[s]``; then dK/dV hop ``s``: this rank's K/V
+    (``kv_slot(0)``) against ``qdo_slot(s)``, the (Q/dO, stat) pair of ``prob.q_owners()[s]``.  A step past the end of
+    one list launches only the other kernel.  ``launched(s)`` follows the launches of step ``s``.
+
+    The fp32 accumulators travel between the launches in carry buffers, and each launch reloads them into TMEM before
+    its first MMA: the launches add the same products in the same order as one launch over every hop, so dQ (and dK /
+    dV without grouped heads) come out bitwise equal to the gather mode."""
+    kv_hops, q_hops = prob.kv_owners(), prob.q_owners()
+    b, h, hk = prob.batch, prob.heads, prob.kv_heads
+    kv_own = kv_slot(0)
+    n_q, d = qdo_own.shape[2], qdo_own.shape[3]
+    n_k = kv_own.shape[2]
+    dev = qdo_own.device
+    none = torch.empty(0, dtype=torch.float32, device=dev)  # a single launch carries nothing
+    dq_carry = torch.empty(b, n_q, h, d, dtype=torch.float32, device=dev) if len(kv_hops) > 1 else none
+    dkv_carry = torch.empty(2, b, n_k, hk, d, dtype=torch.float32, device=dev) if len(q_hops) > 1 else none
+    for s in range(max(len(kv_hops), len(q_hops))):
+        if s < len(kv_hops):
+            kv = kv_own if s == 0 else kv_slot(s)
+            dq = ops.attn_bwd_dq_hop(qdo_own[None], kv[None], stat_own[None], dq_carry, s > 0, s + 1 < len(kv_hops),
+                                     *prob.tail([kv_hops[s]], kmask_bits))
+        if s < len(q_hops):
+            qdo, stat = qdo_slot(s)
+            dk, dv = ops.attn_bwd_dkdv_hop(qdo[None], kv_own[None], stat[None], dkv_carry, s > 0, s + 1 < len(q_hops),
+                                           *prob.tail([q_hops[s]], kmask_bits))
+        launched(s)
+    return dq, dk, dv
+
+
 def emulate_ring_backward(
     qs, ks, vs, outs, lses, douts, *,
     layout: str = "plain",
@@ -225,7 +261,8 @@ def emulate_ring_backward(
     hopwise: bool = False,
 ):
     """Backward of :func:`emulate_ring_forward` for every emulated rank on the current device.
-    ``hopwise`` (fused only): one launch per hop against a single K/V slot (the ``memory="ring"`` schedule).
+    ``hopwise``: one launch per hop (and per kernel of the two-kernel pair) against one-slot views of the gathered
+    buffers (the ``memory="ring"`` schedule).
 
     ``fused`` (default: head dim 128) selects the one-kernel backward: every emulated rank adds its dK / dV tiles into
     the owners' fp32 accumulators, exactly what the ranks of a real ring do over NVLink."""
@@ -281,7 +318,12 @@ def emulate_ring_backward(
             res.append((dq, dk, dv))
         return res
     for r in range(world):
-        # every emulated rank sees the same fully gathered buffers (what the NVLink gather produces)
-        res.append(fused_attn_bwd(AttnProblem(b, h, hk, r, pm, causal, window, scale, softclamp), qdo_all, kv_all,
-                                  stat_all, kbits))
+        prob = AttnProblem(b, h, hk, r, pm, causal, window, scale, softclamp)
+        if hopwise:
+            kv_hops, q_hops = prob.kv_owners(), prob.q_owners()
+            res.append(two_kernel_backward_hops(ops, prob, qdo_all[r], stat_all[r], lambda s: kv_all[kv_hops[s]],
+                                                lambda s: (qdo_all[q_hops[s]], stat_all[q_hops[s]]), kbits))
+        else:
+            # every emulated rank sees the same fully gathered buffers (what the NVLink gather produces)
+            res.append(fused_attn_bwd(prob, qdo_all, kv_all, stat_all, kbits))
     return res

@@ -34,8 +34,16 @@ Backward, head dim 128 (``CONFIG["backward"] = "fused"``):
     once per hop against the 2-slot window ("ring") or once over the gathered slots, which the copy engines re-pull
     behind per-owner flags ("gather") -> device barrier -> fp32 -> 16 bit
 
-Head dim 64 (or ``CONFIG["backward"] = "two_kernel"``): dQ kernel + dK/dV kernel (7 GEMMs, no atomics, deterministic),
-the peers' Q / dO / statistics pulled by the copy engines while the dQ kernel runs.
+Head dim 64 (or ``CONFIG["backward"] = "two_kernel"``): dQ kernel + dK/dV kernel (7 GEMMs, no atomics, deterministic).
+
+    "ring": bwd_prep writes Q / dO / statistics straight into this rank's own symmetric slot, pack_kv re-packs the own
+    K/V slot -> device barrier -> per ring hop one dQ launch (local queries against the K/V of the hop's owner) and one
+    dK/dV launch (local keys against the Q / dO / statistics of the hop's query owner), each against a 2-slot window
+    that the copy engines fill ahead; the fp32 dQ and dK / dV accumulators travel between the launches in carry buffers
+    and are reloaded into TMEM, so the result is bitwise that of the one-launch backward (dK / dV with grouped heads:
+    same sums, another order)
+    "gather": the peers' K/V and Q / dO / statistics gathered into W-slot buffers by the copy engines while the dQ
+    kernel runs
 """
 from __future__ import annotations
 
@@ -58,7 +66,9 @@ from ring_attention_pytorch_b200.ops.fused import (
     fused_attn_bwd_ring,
     fused_attn_fwd,
     pack_key_mask_bits,
+    pad64,
     pad128,
+    two_kernel_backward_hops,
 )
 from ring_attention_pytorch_b200.parallel.distributed import default, exists, get_rank, get_world_size, is_distributed
 from ring_attention_pytorch_b200.parallel.layout import make_position_map
@@ -73,13 +83,13 @@ LAUNCHES = {"count": 0}
 #                        reductions, dK/dV added into the owner's accumulators over NVLink).
 # backward="two_kernel": the dQ + dK/dV kernel pair (7 GEMMs, no atomics, deterministic); head dim 64 always uses it.
 # memory="ring"        : one launch per ring hop against a 2-slot window that the copy engines fill ahead of the
-#                        kernels; the online-softmax state (forward) and the fp32 accumulators (backward, head dim 128)
-#                        carry over between the launches.  Workspace O(n / W) per rank; on par with "gather" at the
-#                        headline size (see the module docstring).
+#                        kernels; the online-softmax state (forward) and the fp32 accumulators (both backwards, every
+#                        head dim) carry over between the launches.  Workspace O(n / W) per rank; on par with "gather"
+#                        at the headline size (see the module docstring).
 # memory="gather"      : one forward launch per rank; its fetcher warps pull all W-1 peer slots into a W-slot gather
 #                        buffer (transient, shared by all layers); workspace O(n) per rank.  Fewer launches: better for
 #                        short shards, where the one-kernel backward's per-launch ramp shows (8 hops x 8192 keys, h=16:
-#                        726 vs 826 TFLOP/s).  The head-dim-64 / two-kernel backward always gathers.
+#                        726 vs 826 TFLOP/s).
 # memory="auto"        : "ring" when one rank's K/V slot is at least AUTO_RING_SLOT_BYTES, else "gather".  Measured on 2
 #                        GPUs: 128 MiB slots (S=16384, h=32) ring 1441 vs gather 1546 TFLOP/s — ~90 us of ramp per extra
 #                        launch against 5 ms steps; 2 GiB slots (S=262144) 1656 vs 1646 (same box, back to back).
@@ -330,8 +340,7 @@ class RingFlashAttentionCUDAFunction(Function):
         hop_owner = prob.kv_owners()
 
         ws, kv_own_ptrs, kv_bytes = None, None, 0
-        hop_mode = (use_ring and d_pad == 128 and CONFIG["backward"] == "fused"
-                    and _use_hop_window(_slot_bytes(b, hk, n_k, d_pad)))
+        hop_mode = use_ring and _use_hop_window(_slot_bytes(b, hk, n_k, d_pad))
         if use_ring:  # re-pack this rank's own slot (the forward's buffers are long reused)
             ws = get_workspace(ring_size, dev)
             own, kv_gather, kv_own_ptrs, kv_bytes = _place_kv(ws, hop_mode, rank, ring_size, b, hk, n_k, d_pad, dt, dev)
@@ -404,6 +413,40 @@ class RingFlashAttentionCUDAFunction(Function):
                     ops.acc_convert(acc[0], dk, 1.0)
                     ops.acc_convert(acc[1], dv, 1.0)
                     _count(3)
+        elif hop_mode:
+            # ---------------- two-kernel backward, one launch per hop and kernel ----------------
+            # bwd_prep writes this rank's Q/dO + statistics straight into its one symmetric slot; after the barrier the
+            # copy engines fill two 2-slot windows: the peers' K/V (for dQ) and their Q/dO + statistics (for dK/dV)
+            n_pad = pad64(n_q)
+            qdo_bytes = 2 * b * h * n_q * d_pad * qp.element_size()
+            qdo_stat_bytes = qdo_bytes + 2 * b * h * n_pad * 4
+            stage, qdo_ptrs = ws.staging("qdo", qdo_stat_bytes)
+            qdo_flat = stage[:qdo_stat_bytes]
+
+            def qdo_stat(flat: Tensor):
+                return (flat[:qdo_bytes].view(dt).view(2, b * h, n_q, d_pad),
+                        flat[qdo_bytes:].view(torch.float32).view(2, b * h, n_pad))
+
+            qdo_own, stat_own = qdo_stat(qdo_flat)
+            with nvtx_range("rab.bwd.prep+barrier"):
+                if n_pad > n_q:  # the dK/dV kernel reads the padding rows (and masks them): keep them finite
+                    stat_own[..., n_q:].zero_()
+                    _count()
+                ops.bwd_prep(qp, o, dop, lse, qdo_own[None], stat_own[None], 0)
+                ws.barrier()  # every peer's own K/V and Q/dO + statistics slots are complete
+                _count(2)
+            with nvtx_range("rab.bwd.kernel"):
+                q_hops = prob.q_owners()
+                kv_window = _HopWindow(ops, ws, own, kv_own_ptrs, kv_bytes, hop_owner)
+                qdo_window = _HopWindow(ops, ws, qdo_flat, qdo_ptrs, qdo_stat_bytes, q_hops)
+
+                def launched(s: int) -> None:
+                    kv_window.launched(s)
+                    qdo_window.launched(s)
+
+                dq, dk, dv = two_kernel_backward_hops(ops, prob, qdo_own, stat_own, kv_window.slot,
+                                                      lambda s: qdo_stat(qdo_window.slot(s)), kbits, launched)
+                _count(len(hop_owner) + len(q_hops))
         else:
             # ---------------- two-kernel backward (csrc/attn_bwd_sm100.cu) ----------------
             qdo_gather = alloc_qdo_buffer(ring_size, b, h, n_q, d_pad, dt, dev)
